@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    (CPU port of the reference path, rank 0 only)
+  python bench.py --steps K --warmup W --dump-outputs DIR  (also writes the results of the last timed step to DIR/*.npy;
+                                                            the inputs are seeded, so two builds can be compared file by file)
 
 One *step* = one complete 100-iteration multi-view SMPLify fit of ONE synthetic sequence of ``--frames`` frames
 (default 10,000 = BASELINE config 3).  STRONG scaling: the sequence is cut into contiguous frame ranges, one per rank
@@ -61,7 +63,14 @@ def parse():
     ap.add_argument('--no-extras', action='store_true', help='skip config4 / config5 / weak / GPU-eager legs')
     ap.add_argument('--cpu-frames', type=int, default=8)
     ap.add_argument('--weak', action='store_true', help='at N>1 also time the weak-scaling run (--frames on every rank)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps write the results of the last one as DIR/<name>.npy (at most 64 MB)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the results of --impl ours; the reference leg times single-frame fits only')
+    return args
 
 
 def peaks():
@@ -234,6 +243,45 @@ def time_events(fn, reps):
         ev[i + 1].record()
     torch.cuda.synchronize()
     return [ev[i].elapsed_time(ev[i + 1]) for i in range(reps)]
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def frame_sample(n_frames, n, seed):
+    """Frames kept in a dump: all of them, or a fixed, seeded sample of ``n`` in frame order."""
+    if n >= n_frames:
+        return np.arange(n_frames)
+    return np.sort(np.random.RandomState(seed).choice(n_frames, max(1, n), replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """``arrays``: name -> device tensor [frames, ...] of a fit's results, in frame order.  Writes out_dir/<name>.npy in
+    float32 / float64, at most DUMP_BYTES in all: the parameters and joints of every frame while they fit into three
+    quarters of it (else a seeded sample of frames), the vertices (126 KB per SMPL-X frame) as a seeded sample of frames in
+    the rest.  frame_index.npy / vertices_frame_index.npy list the frames kept.  Returns the bytes written."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n_frames = len(next(iter(arrays.values())))
+
+    def write(names, budget, seed, index_name):
+        row = sum(arrays[k][0].numel() * arrays[k].element_size() for k in names) + 8      # + the float64 index entry
+        keep = frame_sample(n_frames, budget // row, seed)
+        idx = torch.from_numpy(keep).to(arrays[names[0]].device)
+        out = {index_name: keep.astype(np.float64)}
+        out.update({k: arrays[k].index_select(0, idx).cpu().numpy() for k in names})
+        n = 0
+        for k, a in out.items():
+            if a.dtype not in (np.float32, np.float64):
+                a = a.astype(np.float64)
+            fn = os.path.join(out_dir, k + '.npy')
+            np.save(fn, a)
+            n += os.path.getsize(fn)
+        return n
+    used = write(sorted(k for k in arrays if k != 'vertices'), DUMP_BYTES * 3 // 4, 0, 'frame_index')
+    if 'vertices' in arrays:
+        used += write(['vertices'], DUMP_BYTES - used - 4096, 1, 'vertices_frame_index')      # 4 KB: the two .npy headers
+    return used
 
 
 def kernel_breakdown(pm, sess, F, hbm_peak):
@@ -542,6 +590,15 @@ def run_ours(args):
     sampler.start()
     ms_dev, wall_dev = timed_region(step_device, args.steps, max(args.warmup, 3))
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # what a caller of the timed path holds after its last step: the fitted parameters run() returns and the session's
+        # result tensors (the reference's result-dict keys), every frame of the sequence in frame order
+        res = dict(sess.results(), theta=sess.theta)
+        res = {k: gather_frames(v.contiguous(), F_total) for k, v in res.items()}
+        if rank == 0:
+            nb = dump_outputs(args.dump_outputs, res)
+            log('results of the last timed step: %.1f MB written to %s' % (nb / 1e6, args.dump_outputs))
+        del res
     launches = sess.kernel_launches * args.steps
     ms_e2e, wall_e2e = timed_region(step_e2e, args.steps, max(1, min(args.warmup, 3)))
     h2d, d2h = fit.h2d_bytes, fit.d2h_bytes

@@ -1,11 +1,13 @@
 """ORACLE -- TEST INFRASTRUCTURE ONLY.
 
 Runs the reference's own, UNMODIFIED ``smplify/{smplify,loss,prior}.py`` and
-``models/{smpl,utils}.py`` from /root/reference on the CPU (SURVEY.md Appendix B).
-Works only where /root/reference exists (the authoring container): it is used to
-generate the committed golden vectors (tests/golden/make_golden.py) and to validate
-the standalone restatement ``oracle/fit_port.py``.  Nothing run on the GPU box
-imports this module.
+``models/{smpl,utils}.py`` from a checkout of the reference project on the CPU
+(SURVEY.md Appendix B).  The checkout is the directory named by the environment variable
+BODYFIT_REFERENCE or, when that is unset, a directory ``reference`` beside this
+repository.  Works only where such a checkout exists: it is used to generate the
+committed golden vectors (tests/golden/make_golden*.py) and to validate the standalone
+restatement ``oracle/fit_port.py`` live; without it those live tests skip and the
+golden vectors stand in.  The product and the GPU tests never import this module.
 
 Unrelated imports of the reference are stubbed (torchgeometry, trimesh,
 neural_renderer, matplotlib.dviread, scipy.misc.face, utils.camera, mesh_grid);
@@ -16,8 +18,8 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = '/root/reference'
 _HERE = os.path.dirname(os.path.abspath(__file__))
+REFERENCE_ROOT = os.path.abspath(os.environ.get('BODYFIT_REFERENCE') or os.path.join(_HERE, '..', '..', 'reference'))
 _loaded = {}
 
 
@@ -38,13 +40,13 @@ def load_reference():
     if _loaded:
         return _loaded['ns']
     if not available():
-        raise RuntimeError('reference tree not present at %s' % REFERENCE_ROOT)
+        raise RuntimeError('no reference checkout at %s (set BODYFIT_REFERENCE)' % REFERENCE_ROOT)
     repo = os.path.dirname(_HERE)
     for p in (repo, os.path.join(_HERE, 'shim'), REFERENCE_ROOT):
         if p not in sys.path:
             sys.path.insert(0, p)
     # our package also has sub-packages called models/utils/smplify *inside* bodyfitting_b200,
-    # never top-level, so the reference's top-level names resolve to /root/reference.
+    # never top-level, so the reference's top-level names resolve to the reference checkout.
     nop = lambda *a, **k: None
     if 'torchgeometry' not in sys.modules:
         _stub('torchgeometry', angle_axis_to_rotation_matrix=nop)

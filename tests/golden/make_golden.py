@@ -1,7 +1,7 @@
 """Generates tests/golden/*.npz by running the reference's OWN, unmodified
 smplify/smplify.py (SMPLify.__call__) + smplify/loss.py + smplify/prior.py + models/smpl.py
-from /root/reference on the CPU (oracle/ref_harness.py; smplx arithmetic from the shim).
-Run in the authoring container only:   python tests/golden/make_golden.py
+from a checkout of the reference project on the CPU (oracle/ref_harness.py; smplx arithmetic from the shim):
+    BODYFIT_REFERENCE=<reference checkout> python tests/golden/make_golden.py
 Inputs are the seeded synthetic model / scene of bodyfitting_b200.synthetic (seed 0), so the
 fixtures stay small: only scene inputs and reference outputs are stored, never model tensors.
 """
@@ -22,7 +22,7 @@ def main():
     from bodyfitting_b200 import synthetic as syn
     from oracle import fit_port as fp, ref_harness as rh
     from util import make_scene
-    assert rh.available(), 'needs /root/reference'
+    assert rh.available(), 'needs a checkout of the reference project (BODYFIT_REFERENCE, or reference/ beside the repository)'
     tmp = tempfile.mkdtemp(prefix='bf_golden_')
     syn.write_data_dir(os.path.join(tmp, 'data'), seed=0)
     gmm, jx = syn.make_gmm(0), syn.make_J_regressor_extra(seed=0)

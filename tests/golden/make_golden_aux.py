@@ -1,4 +1,4 @@
-"""Small golden fixtures made by running the reference's OWN code in the authoring container (/root/reference present):
+"""Small golden fixtures made by running the reference's OWN code (BODYFIT_REFERENCE = a checkout of the reference project):
 
   reference_init_conversion.npz  utils/geometry.py:331-493 convert_hom_to_angle (incl. the NaN patch for the identity) and the
                                  world transform of the root orientation, smplify/body_fitting.py:70-73, on seeded rotations;
@@ -6,7 +6,7 @@
                                  openpose/test.json (copied next to it as a data fixture: it is an OpenPose output file, not
                                  reference source).
 
-    python tests/golden/make_golden_aux.py
+    BODYFIT_REFERENCE=<reference checkout> python tests/golden/make_golden_aux.py
 """
 import os
 import shutil

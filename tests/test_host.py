@@ -391,9 +391,10 @@ def test_reference_mesh_grid_wrapper_binds_to_our_module():
     import importlib.util
     import sys
     import types
-    ref = '/root/reference/utils/mesh_grid_searcher.py'
-    if not os.path.exists(ref):
-        pytest.skip('reference tree not present on this machine')
+    from oracle import ref_harness as rh
+    if not rh.available():
+        pytest.skip('no reference checkout (BODYFIT_REFERENCE, or reference/ beside the repository)')
+    ref = os.path.join(rh.REFERENCE_ROOT, 'utils', 'mesh_grid_searcher.py')
     import bodyfitting_b200.compat.mesh_grid as mg
     saved = {k: sys.modules.get(k) for k in ('mesh_grid', 'trimesh')}
     sys.modules['mesh_grid'] = mg
@@ -417,7 +418,7 @@ def test_reference_mesh_grid_wrapper_binds_to_our_module():
 def test_init_conversion_matches_reference_converter():
     """(f)3: rotmat -> axis-angle and the world transform of the root orientation against the REFERENCE'S OWN
     utils/geometry.py:331-493 + smplify/body_fitting.py:70-73 -- committed golden (tests/golden/make_golden_aux.py) and, where
-    /root/reference exists, the live reference functions."""
+    BODYFIT_REFERENCE names a reference checkout, the live reference functions."""
     from bodyfitting_b200.utils.geometry import convert_hom_to_angle, world_init_from_camera_rotmat
     g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_init_conversion.npz'))
     R = torch.tensor(g['rotmat'])

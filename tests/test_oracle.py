@@ -1,6 +1,8 @@
 """CPU tests of the oracle (no GPU): the standalone port against the committed golden vectors
-produced by the verbatim reference, against the verbatim reference itself when /root/reference is
-present, fp32 vs fp64, batched vs per-frame, and finite differences of the LBS restatement."""
+(tests/golden: produced by the verbatim reference; the kid and silhouette paths pinned where the live
+tests held the port equal to it), against the verbatim reference itself where a checkout of it is at
+hand (BODYFIT_REFERENCE, or reference/ beside the repository), fp32 vs fp64, batched vs per-frame, and
+finite differences of the LBS restatement."""
 import os
 
 import numpy as np
@@ -36,7 +38,7 @@ def test_golden_covers_missing_view_and_quirks():
     assert gx['out_joints'].shape == (135, 3) and gx['out_full_pose'].shape == (165,)
 
 
-@pytest.mark.skipif(not rh.available(), reason='/root/reference not present (GPU box)')
+@pytest.mark.skipif(not rh.available(), reason='no reference checkout (BODYFIT_REFERENCE, or reference/ beside the repository)')
 @pytest.mark.parametrize('mt,nv', [('smpl', 4), ('smplx', 8)])
 def test_port_bit_exact_vs_verbatim_reference(assets, tmp_path, mt, nv):
     syn.write_data_dir(str(tmp_path / 'data'), seed=0, model_types=(mt,))
@@ -52,7 +54,7 @@ def test_port_bit_exact_vs_verbatim_reference(assets, tmp_path, mt, nv):
         assert np.array_equal(res[k], resp[k]), k
 
 
-@pytest.mark.skipif(not rh.available(), reason='/root/reference not present (GPU box)')
+@pytest.mark.skipif(not rh.available(), reason='no reference checkout (BODYFIT_REFERENCE, or reference/ beside the repository)')
 def test_kid_model_port_bit_exact_vs_verbatim_reference(assets, tmp_path):
     """age='kid' (smplify/smplify.py:50-56,112-115): the verbatim reference builds SMPL(age='kid', kid_template_path=
     config.SMIL_MODEL_DIR) and starts from 11 zero betas; the restatement follows it bit for bit (the kid shape space itself is
@@ -73,7 +75,7 @@ def test_kid_model_port_bit_exact_vs_verbatim_reference(assets, tmp_path):
         assert np.array_equal(res[k], resp[k]), k
 
 
-@pytest.mark.skipif(not rh.available(), reason='/root/reference not present (GPU box)')
+@pytest.mark.skipif(not rh.available(), reason='no reference checkout (BODYFIT_REFERENCE, or reference/ beside the repository)')
 def test_mask_term_port_bit_exact_vs_verbatim_reference(assets, tmp_path):
     """Silhouette term (use_mask=True, smplify/loss.py:73-130): the restatement run for one frame equals the verbatim
     reference bit for bit (cv2.findContours adapted to OpenCV 4's return arity in the harness)."""
@@ -101,6 +103,41 @@ def test_mask_term_port_bit_exact_vs_verbatim_reference(assets, tmp_path):
     assert mls is not None and (mls > 0).all()
     assert relerr(trb[:N // 3 + 2, 0], np.asarray(trp[:N // 3 + 2])) < 1e-5
     assert relerr(trb[:N // 3 + 3, 0], np.asarray(trp[:N // 3 + 3])) < 1e-3
+
+
+def _fit_golden(port, g, **kw):
+    """One frame of a port_fit_*.npz scene on one torch thread, as the vectors were made (tests/golden/make_golden_port.py:
+    in the mask phase the trajectory follows the last bit of every reduction, which depends on the thread count)."""
+    views = syn.keypoints_to_openpose(g['kp'][0], 'smpl')
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        return port.fit_frame(g['init_betas'][0], g['init_pose'][0], g['c2ws'], g['Ks'], views, num_iters=int(g['num_iters']), **kw)
+    finally:
+        torch.set_num_threads(n)
+
+
+def test_kid_model_port_matches_golden(assets):
+    """The kid path against tests/golden/port_fit_kid.npz: the scene of the live bit-exact test above, stored where that test
+    held the restatement equal to the verbatim reference (tests/golden/make_golden_port.py)."""
+    g = np.load(os.path.join(GOLD, 'port_fit_kid.npz'))
+    port = fp.FitPort('smpl', assets('smpl'), assets('gmm'), assets('jx'), age='kid', kid_template=syn.make_kid_template(0))
+    res, trace = _fit_golden(port, g)
+    assert res['betas'].shape == (11,) and np.abs(res['betas']).max() > 0
+    assert relerr(trace, g['trace']) < 1e-5
+    for k in ('pose', 'betas', 'global_orient', 'global_transl', 'scale', 'joints', 'vertices'):
+        assert np.abs(res[k] - g['out_' + k]).max() < 1e-4, k
+
+
+def test_mask_term_port_matches_golden(assets):
+    """The silhouette term against tests/golden/port_fit_mask.npz: the scene and masks of the live bit-exact test above
+    (tests/golden/make_golden_port.py); the trace includes 5 x the mask term from iteration N//3+1 on."""
+    g = np.load(os.path.join(GOLD, 'port_fit_mask.npz'))
+    port = make_port(assets, 'smpl')
+    res, trace = _fit_golden(port, g, masks=g['masks'], mask_frames=list(g['mask_frames']))
+    assert relerr(trace, g['trace']) < 1e-5
+    for k in ('pose', 'betas', 'global_orient', 'global_transl', 'scale', 'joints', 'vertices', 'full_pose'):
+        assert np.abs(res[k] - g['out_' + k]).max() < 1e-4, k
 
 
 @pytest.mark.parametrize('mt,nv', [('smpl', 4), ('smplx', 8)])
