@@ -777,7 +777,8 @@ int bf_init_theta(const BfModel* m, const float* poses, int ld_poses, const floa
     const int nb = theta_layout(m->is_smplx).nbody;
     BF_REQUIRE(ld_poses >= 3 + nb, "poses need global_orient + body_pose columns");
     const size_t n = (size_t)B * m->NP;
-    k_init_theta<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(poses, ld_poses, betas, theta, B, m->NP, nb, src_index);
+    k_init_theta<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(poses, ld_poses, betas, theta, B, m->NP, nb,
+                                                                                 m->NB < 10 ? m->NB : 10, src_index);
     BF_LAUNCH_CHECK();
     return BF_OK;
 }

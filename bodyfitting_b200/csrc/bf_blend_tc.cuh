@@ -772,15 +772,24 @@ static int bf_blend_forward_tc(const BfModel* m, const BfVSet* vs, const BfFrame
     return bf_gemm_forward_tc(f->pf_hi, f->pf_lo, vs->Bt_hi, vs->Bt_lo, f->B, m->Kp, vs->ldn, vs->n, dst, f->ld_v, s);
 }
 
+// Column tile of the backward GEMM: the widest multiple of 16 (the MMA's N granule) up to 256 that divides Kp.  The kernel
+// streams its operands from L2 and every column tile re-reads the whole dvp row block, so the widest tile wins even when it
+// leaves a partial last wave: measured on 10,000 frames x Kp 512, 64 / 128 / 256 columns = 0.134 / 0.123 / 0.109 ms (158 CTAs
+// on 148 SMs).  Kp = round16(P + NS + 1) is 224 or 240 for SMPL and 512 or 496 for SMPL-X (496 = 16 x 31: NS <= 9, 16-column
+// tiles).  Kp is a multiple of 16 (check_model), so a tile always exists.
+static int bf_bwd_col_tile(int Kp) {
+    for (int bn = Kp < 256 ? Kp : 256; bn > 16; bn -= 16)
+        if (Kp % bn == 0) return bn;
+    return 16;
+}
+
 // The masked backward GEMM always reduces a tile in two halves cut at a fixed block (BW_SPLIT_BLOCK) and adds the two
 // partial sums.  Two forms of the same arithmetic: two CTAs per tile writing dpf and dpf2 (summed by k_pose_bwd), chosen
 // when even the doubled grid is at most one wave -- the batch is small and bound by the latency of one CTA's K loop -- and
 // one CTA per tile with two TMEM accumulators added in its epilogue otherwise (no second buffer to write and re-read).
 static bool bf_bwd_two_cta(const BfModel* m, const BfFrames* f) {
     if (!f->dpf2 || !f->blk_mask || !bf_blk_mask_on()) return false;
-    int BN = m->Kp < 256 ? m->Kp : 256;
-    while (BN > 64 && m->Kp % BN != 0) BN /= 2;
-    if (m->Kp % BN != 0) BN = m->Kp;
+    const int BN = bf_bwd_col_tile(m->Kp);
     const int mt = (f->B + TC_BM - 1) / TC_BM;
     return (m->Kp / BN) * mt * 2 <= bf_num_sms();
 }
@@ -788,16 +797,8 @@ static bool bf_bwd_two_cta(const BfModel* m, const BfFrames* f) {
 static int bf_blend_backward_tc(const BfModel* m, const BfVSet* vs, const BfFrames* f, cudaStream_t s) {
     CUtensorMap a_hi, a_lo, b_hi, b_lo;
     int rc;
-    // column tile: the widest of 256 / 128 / 64 that divides Kp (else Kp itself).  The kernel streams its operands from L2
-    // and every column tile re-reads the whole dvp row block, so the widest tile wins even when it leaves a partial last
-    // wave: measured on 10,000 frames x Kp 512, 64 / 128 / 256 columns = 0.134 / 0.123 / 0.109 ms (158 CTAs on 148 SMs).
     const int num_sms = bf_num_sms();
-    int BN = m->Kp < 256 ? m->Kp : 256;
-    {
-        const int cand[3] = {256, 128, 64};
-        for (int i = 0; i < 3; ++i)
-            if (cand[i] <= m->Kp && m->Kp % cand[i] == 0) { BN = cand[i]; break; }
-    }
+    int BN = bf_bwd_col_tile(m->Kp);                     // the tile bf_bwd_two_cta assumes (narrowed below for small batches)
     if (m->Kp % BN != 0 || BN % 16 != 0) { bf_set_error("Kp=%d not tileable by %d", m->Kp, BN); return BF_EINVAL; }
     // Small batches (a shard of a strong-scaled sequence: 1,250 frames x Kp 512 = 20 tiles of 256 columns on 148 SMs): narrower
     // column tiles until the grid covers at least half of the SMs.  Every output element still accumulates its K products

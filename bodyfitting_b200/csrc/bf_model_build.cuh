@@ -18,6 +18,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -131,6 +132,7 @@ struct Builder {
     int dyn_rows = 0, n_dyn = 0;
     std::vector<JointEntry> joint_table, ori_table;
     const char* err = nullptr;
+    char msg[128] = "";                      // room for an error text with numbers in it (err points here)
 
     explicit Builder(const BfModelDesc& desc) : d(desc) {}
 
@@ -333,8 +335,9 @@ struct Builder {
         }
         for (int j = 1; j < J; ++j) if (d.parents[j] < 0 || d.parents[j] >= j) { err = "kinematic tree must be topologically sorted"; return false; }
         P = (J - 1) * 9;
-        NB = d.num_betas > 0 ? d.num_betas : 10;
-        const int NE = smplx ? (d.num_expression > 0 ? d.num_expression : 10) : 0;
+        NB = d.num_betas;
+        const int NE = smplx ? d.num_expression : 0;
+        if (NB < 1 || NE < 0) { err = "num_betas must be at least 1 and num_expression not negative"; return false; }
         const int S = d.n_shape_dirs;
         vt.assign(d.v_template, d.v_template + (size_t)V * 3);
         // shape directions: [V,3,NB] (+ the kid direction) (+ NE expression directions; official files keep them after 300)
@@ -366,6 +369,10 @@ struct Builder {
         const int Kdim = P + NS + 1;
         Kp = round_up(Kdim, 16);
         NP = 7 + (smplx ? 63 : 69) + NB + (smplx ? 18 : 0);
+        // the kernels' per-frame limits (BF_MAXNS / BF_MAXNP), checked here so that such a model fails when it is built rather
+        // than at its first launch; the Python builder raises the same text
+        if (NS > BF_MAXNS) { snprintf(msg, sizeof(msg), "%d shape coefficients (betas + expression) exceed the limit of %d", NS, BF_MAXNS); err = msg; return false; }
+        if (NP > BF_MAXNP) { snprintf(msg, sizeof(msg), "%d theta entries exceed the limit of %d", NP, BF_MAXNP); err = msg; return false; }
 
         // kinematic tree
         std::vector<int32_t> parents(J), depth(J, 0), child_ptr(J + 1, 0), child_idx;

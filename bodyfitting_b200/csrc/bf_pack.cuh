@@ -5,7 +5,8 @@
 //                      confidences as [N,1], which broadcasts against the [N] residuals, so every joint of such a group
 //                      weighs sum_i conf_i^2 of that group and view (smplify/loss.py:134 with :168,:173,:179).
 //   k_init_theta     : network output (betas [B,10], poses [B,>=3+nbody]) -> theta rows: transl 0, scale 1, global
-//                      orient / body pose / betas from the network, eyes / hands 0 (smplify/smplify.py:103-128).
+//                      orient / body pose / betas from the network, eyes / hands 0 (smplify/smplify.py:103-128).  A model
+//                      with more than 10 betas (the kid model) starts the others at 0; one with fewer takes the first NB.
 //   halo             : the temporal term couples frame f with f-1 / f+1; across shards the boundary rows live on the
 //                      neighbouring GPUs.  Each rank owns one small cudaMalloc'ed buffer (exported by CUDA IPC, mapped by
 //                      its neighbours); a rank WRITES its boundary theta rows straight into the neighbours' buffers over
@@ -98,7 +99,7 @@ __global__ void __launch_bounds__(256) k_pack_keypoints(const float* __restrict_
 }
 
 __global__ void __launch_bounds__(256) k_init_theta(const float* __restrict__ poses, int ldp, const float* __restrict__ betas,
-                                                    float* __restrict__ theta, int B, int NP, int nbody,
+                                                    float* __restrict__ theta, int B, int NP, int nbody, int nbeta_in,
                                                     const int32_t* __restrict__ src_index) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)B * NP) return;
@@ -107,7 +108,7 @@ __global__ void __launch_bounds__(256) k_init_theta(const float* __restrict__ po
     float v = 0.f;
     if (c == 3) v = 1.0f;                                                      // body_scale
     else if (c >= 4 && c < 7 + nbody) v = poses[(size_t)b * ldp + (c - 4)];    // global_orient | body_pose
-    else if (c >= 7 + nbody && c < 17 + nbody) v = betas[(size_t)b * 10 + (c - 7 - nbody)];
+    else if (c >= 7 + nbody && c < 7 + nbody + nbeta_in) v = betas[(size_t)b * 10 + (c - 7 - nbody)];
     theta[i] = v;
 }
 

@@ -406,10 +406,11 @@ __global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int fla
 
     // betas: rest-joint path + shape rows of the blend GEMM
     {
-        // lanes (l, part): 3 parts (2 when more than 10 betas: the kid model) split the 3J rest-joint coordinates, combined
-        // in a fixed order
+        // lanes (l, part): the 3J rest-joint coordinates are split into as many parts as fit into the warp -- 3 up to 10
+        // betas, 2 up to 16 (the kid model), 1 above -- and combined in a fixed order.  Lane l + NB * part must stay below
+        // 32: a part beyond that would wrap around the shuffles below and add another beta's partial sum.
         const int l = lane % m.NB, part = lane / m.NB;
-        const int nparts = 3 * m.NB <= 32 ? 3 : 2;
+        const int nparts = 3 * m.NB <= 32 ? 3 : 2 * m.NB <= 32 ? 2 : 1;
         const int nq = 3 * J, per = (nq + nparts - 1) / nparts;
         float acc = 0.f;
         if (part < nparts) {
@@ -417,8 +418,9 @@ __global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int fla
 #pragma unroll 11
             for (int q = part * per; q < q1; ++q) acc += __ldg(m.Jd + q * m.NS + l) * dJr_s[q];
         }
-        const float a1 = __shfl_sync(0xffffffffu, acc, (lane + m.NB) & 31);
+        const float a1s = __shfl_sync(0xffffffffu, acc, (lane + m.NB) & 31);
         const float a2s = __shfl_sync(0xffffffffu, acc, (lane + 2 * m.NB) & 31);
+        const float a1 = nparts > 1 ? a1s : 0.f;
         const float a2 = nparts > 2 ? a2s : 0.f;
         if (lane < m.NB) {
             float dsh = f.dpf[(size_t)b * m.Kp + m.P + lane];

@@ -31,6 +31,10 @@ from . import _lib
 from . import constants as K
 
 
+MAX_NS = 20         # betas + expression coefficients per frame (BF_MAXNS, csrc/bf_common.cuh)
+MAX_NP = 100        # theta entries per frame (BF_MAXNP)
+
+
 def _round_up(x, m):
     return (x + m - 1) // m * m
 
@@ -137,6 +141,8 @@ class PreparedModel(object):
         J = len(parents)
         assert all(parents[j] < j for j in range(1, J)), 'kinematic tree must be topologically sorted'
         P = (J - 1) * 9
+        if num_betas < 1 or (self.is_smplx and num_expression < 0):
+            raise ValueError('num_betas must be at least 1 and num_expression not negative')
         NB = num_betas
         sd_all = np.asarray(data['shapedirs'], dtype=np.float32)
         if sd_all.ndim == 2:
@@ -160,6 +166,13 @@ class PreparedModel(object):
         elif age != 'adult':
             raise ValueError("age must be 'adult' or 'kid'")
         NS = NB + (num_expression if self.is_smplx else 0)
+        NP = 7 + (63 if self.is_smplx else 69) + NB + (18 if self.is_smplx else 0)      # 98 / 86 (87 for the kid model)
+        # the kernels' per-frame limits, checked when the model is built rather than at its first launch (same text as the
+        # C++ builder, csrc/bf_model_build.cuh)
+        if NS > MAX_NS:
+            raise ValueError('%d shape coefficients (betas + expression) exceed the limit of %d' % (NS, MAX_NS))
+        if NP > MAX_NP:
+            raise ValueError('%d theta entries exceed the limit of %d' % (NP, MAX_NP))
         if self.is_smplx and sd_all.shape[-1] >= K.SHAPE_SPACE_DIM + num_expression:
             # official files: the expression directions follow the 300 shape directions (smplx: SHAPE_SPACE_DIM)
             sd = np.concatenate([sd_all[:, :, :NB], sd_all[:, :, K.SHAPE_SPACE_DIM:K.SHAPE_SPACE_DIM + num_expression]], -1)
@@ -174,7 +187,7 @@ class PreparedModel(object):
         self.V, self.J, self.P, self.NB, self.NS = V, J, P, NB, NS
         self.Kdim = P + NS + 1
         self.Kp = _round_up(self.Kdim, 16)
-        self.NP = 7 + (63 if self.is_smplx else 69) + NB + (18 if self.is_smplx else 0)      # 98 / 86 (87 for the kid model)
+        self.NP = NP
         self.nbody = 63 if self.is_smplx else 69
         self.parents = parents
 

@@ -255,6 +255,8 @@ typedef struct BfModelDesc {
     const float*   gmm_means;               /* [n_gmm,69]   pose prior (smplify/prior.py:127), or NULL */
     const float*   gmm_covars;              /* [n_gmm,69,69] */
     const float*   gmm_weights;             /* [n_gmm] */
+    /* num_betas >= 1 (the kid template adds one more); num_expression >= 0 (SMPL-X only; 0 = no expression directions).
+     * The model is rejected when betas + expression exceed 20 or its theta row exceeds 100 entries (NP above). */
     int32_t is_smplx, V, J, F, n_shape_dirs, num_betas, num_expression, n_lmk, n_dyn_rows, n_dyn, n_extra_vids, n_regressor_extra,
             n_gmm, tensor_cores, _pad0, _pad1;
 } BfModelDesc;
@@ -278,7 +280,9 @@ int bf_graph_set_kernel_priority(void* cuda_graph, int priority);
 int bf_pack_keypoints(const float* kp_raw, float* kp_packed, int B, int Nv, int K, int hand_face, const int32_t* src_index,
                       void* stream);
 /* network output -> initial theta rows (smplify/smplify.py:103-128): transl 0, scale 1, global_orient / body_pose from
- * poses[b, 0:3+nbody] (row stride ld_poses), betas[b, 0:10], eye / hand parameters 0 */
+ * poses[b, 0:3+nbody] (row stride ld_poses), betas[b, 0:10], eye / hand parameters 0.  betas always has 10 columns: a model
+ * with more betas (num_betas > 10, the kid model) starts the betas beyond the 10th at 0, one with fewer takes the first
+ * num_betas columns.  To start them elsewhere, write the theta rows directly (layout at the top of this file). */
 int bf_init_theta(const BfModel* m, const float* poses, int ld_poses, const float* betas, float* theta, int B,
                   const int32_t* src_index, void* stream);
 /* src_index (both calls above, optional): packed frame b is the caller's frame src_index[b] -- a batch whose frames are

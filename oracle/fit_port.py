@@ -110,14 +110,17 @@ class _Mapper(nn.Module):
         return torch.index_select(joints, 1, self.idx)
 
 
-def build_model(smpl_type, model_data, J_regressor_extra=None, dtype=torch.float32, age='adult', kid_template=''):
-    """Body model exactly as SMPLify.__init__ builds it (smplify/smplify.py:50-80)."""
+def build_model(smpl_type, model_data, J_regressor_extra=None, dtype=torch.float32, age='adult', kid_template='',
+                num_betas=10, num_expression=10):
+    """Body model exactly as SMPLify.__init__ builds it (smplify/smplify.py:50-80); ``num_betas`` / ``num_expression`` (SMPL-X)
+    select other shape-space sizes (the reference uses smplx's defaults, 10 / 10)."""
     if smpl_type == 'smpl':
-        m = SpinSMPL(model_data, J_regressor_extra, dtype=dtype, age=age, kid_template_path=kid_template)
+        m = SpinSMPL(model_data, J_regressor_extra, dtype=dtype, age=age, kid_template_path=kid_template, num_betas=num_betas)
     else:
         mapper = _Mapper(C.smpl_to_openpose('smplx', use_hands=True, use_face=True, use_face_contour=True,
                                             openpose_format='coco25'))
-        m = sp.SMPLXLayer(model_data, joint_mapper=mapper, use_face_contour=True, create_transl=False, dtype=dtype)
+        m = sp.SMPLXLayer(model_data, num_betas=num_betas, num_expression_coeffs=num_expression, joint_mapper=mapper,
+                          use_face_contour=True, create_transl=False, dtype=dtype)
     return m
 
 
@@ -243,16 +246,20 @@ def batched_objective(w2cs, Ks, kp, model_joints, poses, betas, prior, imsize, u
 
 class FitPort(object):
     def __init__(self, smpl_type, model_data, gmm, J_regressor_extra=None, dtype=torch.float32,
-                 constant_scale=C.CONSTANT_SCALE_NO_SCAN, device='cpu', age='adult', kid_template=''):
+                 constant_scale=C.CONSTANT_SCALE_NO_SCAN, device='cpu', age='adult', kid_template='', num_betas=10,
+                 num_expression=10):
         """``device='cuda'``: the same eager op sequence on the GPU (the reference's default device, smplify.py:29) --
-        bench.py's second, non-target baseline; parity is always checked with the CPU path."""
+        bench.py's second, non-target baseline; parity is always checked with the CPU path.  ``num_betas`` /
+        ``num_expression``: shape-space sizes of the body model (build_model)."""
         self.smpl_type = smpl_type
         self.use_hand_face = smpl_type == 'smplx'
         self.dtype = dtype
         self.device = torch.device(device)
         self.prior = GMMPrior(gmm, dtype=dtype).to(self.device)
         self.age = age
-        self.model = build_model(smpl_type, model_data, J_regressor_extra, dtype=dtype, age=age, kid_template=kid_template).to(self.device)
+        self.model = build_model(smpl_type, model_data, J_regressor_extra, dtype=dtype, age=age, kid_template=kid_template,
+                                 num_betas=num_betas, num_expression=num_expression).to(self.device)
+        self.num_betas = self.model.num_betas          # the kid model: num_betas + 1
         if hasattr(self.model, 'joint_map'):
             self.model.joint_map = self.model.joint_map.to(self.device)
         self.constant_scale = constant_scale
@@ -265,7 +272,7 @@ class FitPort(object):
         nb = 69 if self.smpl_type == 'smpl' else 63
         p = dict(body_pose=init_poses[:, 3:3 + nb].detach().clone(),
                  betas=(torch.as_tensor(init_betas, dtype=dt).reshape(B, -1).to(dev).detach().clone() if self.age == 'adult'
-                        else torch.zeros(B, 11, dtype=dt, device=dev)),            # smplify.py:112-115
+                        else torch.zeros(B, self.num_betas, dtype=dt, device=dev)),     # smplify.py:112-115
                  global_orient=init_poses[:, :3].detach().clone(),
                  global_transl=torch.zeros(B, 3, dtype=dt, device=dev), body_scale=torch.ones(B, 1, dtype=dt, device=dev),
                  jaw_pose=torch.zeros(B, 1, 3, dtype=dt, device=dev), leye_pose=torch.zeros(B, 1, 3, dtype=dt, device=dev),

@@ -523,12 +523,25 @@ def _parse_blob(raw):
     return img, {k: sec[o:ends[ends.index(o) + 1]] for k, o in offs.items()}
 
 
-@pytest.mark.parametrize('case', ['smpl', 'smplx', 'smpl_kid', 'smpl_plain', 'smplx_official'])
+# other shape-space sizes: (model type, num_betas, num_expression), the kid template adds one beta.  The same grid as
+# tests/test_gpu_model_shapes.py: 1 / 16 / 17 / 20 betas, NS = 20 with NP = 100, no expression at all, Kp = 496 (NS <= 9)
+_COUNTS = {'smpl_nb1': ('smpl', 1, 0), 'smpl_nb16': ('smpl', 16, 0), 'smpl_nb17': ('smpl', 17, 0), 'smpl_nb20': ('smpl', 20, 0),
+           'smpl_kid_nb16': ('smpl', 16, 0), 'smplx_nb12_ne8': ('smplx', 12, 8), 'smplx_nb10_ne0': ('smplx', 10, 0),
+           'smplx_nb5_ne4': ('smplx', 5, 4), 'smplx_nb1_ne0': ('smplx', 1, 0)}
+
+
+@pytest.mark.parametrize('case', ['smpl', 'smplx', 'smpl_kid', 'smpl_plain', 'smplx_official'] + list(_COUNTS))
 def test_bf_model_create_tables_match_python_builder(assets, case, tmp_path):
     """include/bodyfit_b200.h: bf_model_build_blob (what bf_model_create uploads) builds the SAME tables from the raw model
-    arrays as bodyfitting_b200.model.PreparedModel: index tables bit for bit; folded / inverted float tables to rounding."""
+    arrays as bodyfitting_b200.model.PreparedModel: index tables bit for bit; folded / inverted float tables to rounding --
+    for the default shape space and for other numbers of betas / expression coefficients."""
     mt = 'smplx' if case.startswith('smplx') else 'smpl'
     model = assets(mt)
+    counts = {}
+    if case in _COUNTS:
+        _, nb, ne = _COUNTS[case]
+        model = syn.make_model(mt, 0, nb, ne)
+        counts = dict(num_betas=nb, num_expression=ne)
     if case == 'smplx_official':
         # the layout of the official files: no 'extra_vids' key (smplx hard-codes the ids), 300 shape + 100 expression directions
         model = {k: v for k, v in model.items() if k != 'extra_vids'}
@@ -537,17 +550,18 @@ def test_bf_model_create_tables_match_python_builder(assets, case, tmp_path):
         wide[:, :, :10], wide[:, :, 300:310] = sd[:, :, :10], sd[:, :, 10:20]
         wide[:, :, 10:300] = 1e-3                                      # directions the fit must not pick up
         model['shapedirs'] = wide
-    kw = {}
-    if case == 'smpl_kid':
-        kw = dict(kid_template=syn.make_kid_template(0))
-    jx = assets('jx') if case in ('smpl', 'smpl_kid') else None
+    kid = case.startswith('smpl_kid')
+    kw = dict(kid_template=syn.make_kid_template(0)) if kid else {}
+    jx = assets('jx') if (mt == 'smpl' and case != 'smpl_plain') else None
     gmm = None if case == 'smpl_plain' else assets('gmm')
     pm = PreparedModel(mt, model, gmm=gmm, J_regressor_extra=jx, device='cpu', tensor_cores=True,
-                       age='kid' if case == 'smpl_kid' else 'adult', **kw)
+                       age='kid' if kid else 'adult', **kw, **counts)
+    if counts:
+        assert pm.NB == counts['num_betas'] + kid and pm.NS == pm.NB + (counts['num_expression'] if mt == 'smplx' else 0)
     path = pm.save_blob(str(tmp_path / 'py.blob'))
     img_p, arr_p = _parse_blob(open(path, 'rb').read())
     from bodyfitting_b200.model import model_desc
-    d, keep = model_desc(mt, model, gmm=gmm, J_regressor_extra=jx, tensor_cores=True, **kw)
+    d, keep = model_desc(mt, model, gmm=gmm, J_regressor_extra=jx, tensor_cores=True, **kw, **counts)
     assert (d.extra_vids is None) == (case == 'smplx_official')
     blob, n = ctypes.c_void_p(), ctypes.c_int64()
     rc = _lib.lib().bf_model_build_blob(ctypes.byref(d), ctypes.byref(blob), ctypes.byref(n))
@@ -631,3 +645,47 @@ def test_bf_model_create_rejects_bad_descriptions(assets):
     d.kid_template = kid.ctypes.data
     rc, msg = build(d)
     assert rc != 0 and 'SMPL only' in msg
+
+
+def test_builders_agree_on_shape_space_limits(assets):
+    """Both model builders (bf_model_build_blob in C++ and PreparedModel in Python) reject, with the same text, shape spaces the
+    kernels cannot run: more than 20 betas + expression coefficients (BF_MAXNS), more than 100 theta entries (BF_MAXNP), or
+    fewer than one beta -- when the model is built, not at its first launch.  Zero expression coefficients are honoured by
+    both (SMPL-X without expression directions)."""
+    from bodyfitting_b200.model import model_desc
+    L = _lib.lib()
+
+    def both(mt, nb, ne, **kw):
+        data = syn.make_model(mt, 0, max(nb, 1), max(ne, 0))
+        d, keep = model_desc(mt, data, num_betas=nb, num_expression=ne, **kw)
+        blob, n = ctypes.c_void_p(), ctypes.c_int64()
+        rc = L.bf_model_build_blob(ctypes.byref(d), ctypes.byref(blob), ctypes.byref(n))
+        img = None
+        if rc == 0:
+            img, _ = _parse_blob(ctypes.string_at(blob, n.value))
+            L.bf_blob_free(blob)
+        c = (rc, None if rc == 0 else _lib.last_error(), img)
+        try:
+            pm = PreparedModel(mt, data, device='cpu', tensor_cores=False, num_betas=nb, num_expression=ne,
+                               age='kid' if 'kid_template' in kw else 'adult', **kw)
+            return c, (None, pm)
+        except ValueError as e:
+            return c, (str(e), None)
+
+    kid = dict(kid_template=syn.make_kid_template(0))
+    for mt, nb, ne, kw, text in (('smplx', 16, 4, {}, '104 theta entries exceed the limit of 100'),      # NS = 20, NP = 104
+                                 ('smplx', 12, 9, {}, '21 shape coefficients (betas + expression) exceed the limit of 20'),
+                                 ('smpl', 21, 0, {}, '21 shape coefficients (betas + expression) exceed the limit of 20'),
+                                 ('smpl', 20, 0, kid, '21 shape coefficients (betas + expression) exceed the limit of 20'),
+                                 ('smpl', 0, 0, {}, 'num_betas must be at least 1 and num_expression not negative'),
+                                 ('smplx', 0, 10, {}, 'num_betas must be at least 1 and num_expression not negative'),
+                                 ('smplx', 10, -1, {}, 'num_betas must be at least 1 and num_expression not negative')):
+        (rc, cmsg, _), (pmsg, _) = both(mt, nb, ne, **kw)
+        assert rc != 0 and cmsg.endswith(text), (mt, nb, ne, cmsg)
+        assert pmsg == text, (mt, nb, ne, pmsg)
+    # the largest accepted shape spaces, and SMPL-X without expression: both builders take the counts as given
+    for mt, nb, ne, kw, ns, np_ in (('smplx', 12, 8, {}, 20, 100), ('smpl', 20, 0, {}, 20, 96), ('smpl', 19, 0, kid, 20, 96),
+                                    ('smplx', 10, 0, {}, 10, 98), ('smplx', 1, 0, {}, 1, 89)):
+        (rc, cmsg, img), (pmsg, pm) = both(mt, nb, ne, **kw)
+        assert rc == 0 and pmsg is None, (mt, nb, ne, cmsg, pmsg)
+        assert (img.NS, img.NP) == (pm.NS, pm.NP) == (ns, np_), (mt, nb, ne)
