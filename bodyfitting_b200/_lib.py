@@ -10,7 +10,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('BODYFIT_LIB') or os.path.join(_HERE, 'libbodyfit_b200.so')   # BODYFIT_LIB: A/B builds of the same ABI
-ABI_VERSION = 19
+ABI_VERSION = 20
 F_WORLD = 1
 F_TC = 2
 F_SKIN_FUSED = 4
@@ -34,7 +34,7 @@ class BfModelDesc(C.Structure):
         'hands_componentsl', 'hands_componentsr', 'lmk_faces_idx', 'lmk_bary_coords', 'dynamic_lmk_faces_idx',
         'dynamic_lmk_bary_coords', 'extra_vids', 'J_regressor_extra', 'kid_template', 'gmm_means', 'gmm_covars', 'gmm_weights')] + \
         [(n, _i32) for n in ('is_smplx', 'V', 'J', 'F', 'n_shape_dirs', 'num_betas', 'num_expression', 'n_lmk', 'n_dyn_rows', 'n_dyn',
-                             'n_extra_vids', 'n_regressor_extra', 'n_gmm', 'tensor_cores', '_pad0', '_pad1')]
+                             'n_extra_vids', 'n_regressor_extra', 'n_gmm', 'tensor_cores', 'face_params', '_pad1')]
 
 
 class BfModel(C.Structure):
@@ -43,7 +43,7 @@ class BfModel(C.Structure):
         'gmm_mean', 'gmm_psym', 'gmm_logw', 'gmm_bt_hi', 'gmm_bt_lo')] + \
         [('full', BfVSet), ('act', BfVSet)] + \
         [(n, _i32) for n in ('J', 'P', 'NS', 'NB', 'Kp', 'NP', 'is_smplx', 'max_depth', 'K_used',
-                             'n_gmm', '_pad0', '_pad1')]
+                             'n_gmm', 'face', '_pad1')]
 
 
 class BfFrames(C.Structure):
@@ -53,7 +53,7 @@ class BfFrames(C.Structure):
         'pf_hi', 'pf_lo', 'dvp_hi', 'dvp_lo', 'gmm_grad', 'gmm_loss', 'tgrad', 'tloss', 'halo_prev', 'halo_next', 'halo_buf', 'halo_peer_prev', 'halo_peer_next', 'fwd_state', 'gmm_ws', 'ws', 'blk_mask', 'dpf2', 'frame_index')] + [('ws_floats', C.c_int64)] + \
         [(n, C.c_double) for n in ('lr_ts', 'lr', 'beta1', 'beta2', 'eps')] + \
         [(n, _i32) for n in ('B', 'Nv', 'ld_v', 'iter', 'flags', 'halo_iters')] + \
-        [(n, C.c_float) for n in ('imsize', 'constant_scale', 'sigma', 'w_pose', 'w_angle', 'w_shape', 'w_temporal', '_padf')]
+        [(n, C.c_float) for n in ('imsize', 'constant_scale', 'sigma', 'w_pose', 'w_angle', 'w_shape', 'w_temporal', 'w_expr')]
 
 
 class BfGrid(C.Structure):

@@ -24,6 +24,7 @@ FACE_MAPPING = list(range(17, 17 + 51)) + list(range(0, 17))   # smplify/loss.py
 
 GMOF_SIGMA = 100.0            # smplify/loss.py:139
 SHAPE_PRIOR_WEIGHT = 5.0      # smplify/loss.py:140
+EXPR_PRIOR_WEIGHT = 5.0       # expression L2 prior of face-parameter fits (this project's choice; not in the reference)
 ANGLE_PRIOR_WEIGHT = 15.2     # smplify/loss.py:140
 POSE_PRIOR_WEIGHT = 4.78      # smplify/loss.py:141
 ANGLE_PRIOR_IDXS = [52, 55, 9, 12]            # smplify/loss.py:60-61 (into the 69-D body pose)

@@ -34,7 +34,9 @@ static int check_model(const BfModel* m, const BfFrames* f) {
     BF_REQUIRE(m && f, "null model / frames");
     BF_REQUIRE(m->J > 0 && m->J <= BF_MAXJ, "J out of range");
     BF_REQUIRE(m->NS > 0 && m->NS <= BF_MAXNS && m->NB <= m->NS, "NS/NB out of range");
-    BF_REQUIRE(m->NP == theta_layout(m->is_smplx, m->NB).np && m->NP <= BF_MAXNP, "NP does not match theta layout");
+    BF_REQUIRE(m->face == 0 || (m->face == 1 && m->is_smplx), "face parameters apply to SMPL-X only");
+    BF_REQUIRE(m->NP == theta_layout(*m).np && theta_layout(m->is_smplx, m->NB).np <= BF_MAXNP && m->NP <= BF_THETA_SMEM,
+               "NP does not match theta layout");
     BF_REQUIRE(m->Kp % 16 == 0 && m->Kp >= m->P + m->NS + 1, "Kp must be a multiple of 16 covering P+NS+1");
     BF_REQUIRE(m->P == (m->J - 1) * 9, "P != 9(J-1)");
     BF_REQUIRE(m->parents && m->lvl_ptr && m->lvl_j && m->child_ptr && m->child_idx, "kinematic tree tables missing");
@@ -710,6 +712,7 @@ static void carve_frames(const BfModel* m, int B, int Nv, int opts, int n_trace,
     // defaults), loss.py:139-141 (sigma 100, prior weights 4.78 / 15.2 / 5)
     f->lr_ts = 0.1; f->lr = 1e-2; f->beta1 = 0.9; f->beta2 = 0.999; f->eps = 1e-8;
     f->imsize = 512.f; f->constant_scale = 0.3f; f->sigma = 100.f; f->w_pose = 4.78f; f->w_angle = 15.2f; f->w_shape = 5.f;
+    f->w_expr = 5.f;                                  // expression prior of face models (this project's default)
 }
 
 int64_t bf_workspace_bytes(const BfModel* m, int B, int Nv, int opts, int n_trace) {

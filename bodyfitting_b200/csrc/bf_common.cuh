@@ -9,7 +9,8 @@
 
 #define BF_MAXJ 55          // SMPL-X kinematic tree
 #define BF_MAXNS 20         // 10 betas + 10 expression coefficients
-#define BF_MAXNP 100        // theta entries (86 / 98)
+#define BF_MAXNP 100        // theta entries without the face block (86 / 98)
+#define BF_THETA_SMEM 112   // per-frame theta storage: a face-parameter row adds 3 + NE <= 23 entries (at most 111)
 #define BF_GMM_D 69
 
 void bf_set_error(const char* fmt, ...);
@@ -65,10 +66,11 @@ struct BfRange {
 
 // theta layout (see include/bodyfit_b200.h)
 struct ThetaLayout {
-    int nbody, off_betas, off_leye, off_reye, off_lh, off_rh, np;
+    int nbody, off_betas, off_leye, off_reye, off_lh, off_rh, off_jaw, off_expr, np;
 };
 // nbetas: 10, or 11 for the SMPL kid model (age='kid': the SMIL template difference is an extra shape direction)
-__host__ __device__ __forceinline__ ThetaLayout theta_layout(int is_smplx, int nbetas = 10) {
+// face (SMPL-X only): the row ends with [jaw 3 | expression nexpr]; without it off_jaw = off_expr = np
+__host__ __device__ __forceinline__ ThetaLayout theta_layout(int is_smplx, int nbetas = 10, int face = 0, int nexpr = 0) {
     ThetaLayout t;
     t.nbody = is_smplx ? 63 : 69;
     t.off_betas = 7 + t.nbody;
@@ -76,8 +78,13 @@ __host__ __device__ __forceinline__ ThetaLayout theta_layout(int is_smplx, int n
     t.off_reye = t.off_leye + 3;
     t.off_lh = t.off_reye + 3;
     t.off_rh = t.off_lh + 6;
-    t.np = is_smplx ? t.off_rh + 6 : t.off_betas + nbetas;
+    t.off_jaw = is_smplx ? t.off_rh + 6 : t.off_betas + nbetas;
+    t.off_expr = t.off_jaw + ((is_smplx && face) ? 3 : 0);
+    t.np = t.off_expr + ((is_smplx && face) ? nexpr : 0);
     return t;
+}
+__host__ __device__ __forceinline__ ThetaLayout theta_layout(const BfModel& m) {
+    return theta_layout(m.is_smplx, m.NB, m.face, m.NS - m.NB);
 }
 
 // round-to-nearest TF32 (10-bit mantissa, low 13 bits zero) and the exact fp32 remainder: x = hi + lo

@@ -338,6 +338,8 @@ struct Builder {
         NB = d.num_betas;
         const int NE = smplx ? d.num_expression : 0;
         if (NB < 1 || NE < 0) { err = "num_betas must be at least 1 and num_expression not negative"; return false; }
+        if (d.face_params && !smplx) { err = "face parameters (jaw pose, expression) apply to SMPL-X only"; return false; }
+        const bool face = smplx && d.face_params != 0;
         const int S = d.n_shape_dirs;
         vt.assign(d.v_template, d.v_template + (size_t)V * 3);
         // shape directions: [V,3,NB] (+ the kid direction) (+ NE expression directions; official files keep them after 300)
@@ -370,9 +372,11 @@ struct Builder {
         Kp = round_up(Kdim, 16);
         NP = 7 + (smplx ? 63 : 69) + NB + (smplx ? 18 : 0);
         // the kernels' per-frame limits (BF_MAXNS / BF_MAXNP), checked here so that such a model fails when it is built rather
-        // than at its first launch; the Python builder raises the same text
+        // than at its first launch; the Python builder raises the same text.  The 100-entry limit applies to the row without
+        // the face block; that block (3 + NE entries) is bounded by the shape limit, so a face row has at most 111 entries.
         if (NS > BF_MAXNS) { snprintf(msg, sizeof(msg), "%d shape coefficients (betas + expression) exceed the limit of %d", NS, BF_MAXNS); err = msg; return false; }
         if (NP > BF_MAXNP) { snprintf(msg, sizeof(msg), "%d theta entries exceed the limit of %d", NP, BF_MAXNP); err = msg; return false; }
+        if (face) NP += 3 + NE;                          // [jaw 3 | expression NE] after the right-hand PCA
 
         // kinematic tree
         std::vector<int32_t> parents(J), depth(J, 0), child_ptr(J + 1, 0), child_idx;
@@ -554,7 +558,7 @@ struct Builder {
         std::vector<JointEntry> act_table(joint_table.begin(), joint_table.begin() + K_used);
         if (!build_vset(active, act_table, true, &m->act)) return false;
         m->J = J; m->P = P; m->NS = NS; m->NB = NB; m->Kp = Kp; m->NP = NP; m->is_smplx = smplx ? 1 : 0;
-        m->max_depth = max_depth; m->K_used = K_used; m->n_gmm = n_gmm;
+        m->max_depth = max_depth; m->K_used = K_used; m->n_gmm = n_gmm; m->face = face ? 1 : 0;
         return true;
     }
 };

@@ -18,7 +18,7 @@
 #pragma once
 #include "bf_common.cuh"
 
-#define BF_HALO_ROW 128                      // floats per boundary row slot (NP <= 100)
+#define BF_HALO_ROW 128                      // floats per boundary row slot (NP <= 111)
 #define BF_HALO_PREV 0                       // [2][128] rows written by rank-1 (its LAST frame)
 #define BF_HALO_NEXT (2 * BF_HALO_ROW)       // [2][128] rows written by rank+1 (its FIRST frame)
 #define BF_HALO_FLAGS (4 * BF_HALO_ROW)      // uint32: flag_prev[2], flag_next[2]

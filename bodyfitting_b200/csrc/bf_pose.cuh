@@ -5,6 +5,8 @@
 //   k_pose_bwd : recompute the above in shared memory, reverse chain traversal,
 //                Rodrigues backward, PCA-hand backward, GMM / angle / shape priors and the
 //                Adam update, fused per frame.
+// A face-parameter SMPL-X model (BfModel.face) also carries the jaw pose and the expression coefficients in theta: the forward
+// takes them into the full pose / shape row, the backward produces their gradients (+ the expression L2 prior) and Adam steps them.
 // Replaces smplx batch_rodrigues + batch_rigid_transform (restated in oracle/smplx_port.py),
 // smplify/prior.py:181-196, smplify/loss.py:54-61,206-217 and torch.optim.Adam
 // (smplify/smplify.py:167-174,211-213).
@@ -12,10 +14,11 @@
 #include "bf_common.cuh"
 #include "bf_pack.cuh"
 
-// fp | R | Jr | GR are contiguous and 16-byte aligned, in the order of a saved forward-state row ([fp 3J | R 9J | Jr 3J |
-// GR 9J], pose_write_outputs): for J == BF_MAXJ the backward fetches the row with ONE bulk copy.
-struct __align__(16) PoseSmem {
-    float th[BF_MAXNP];
+// fp | R | Jr | GR are contiguous and 16-byte aligned (in PoseSmemBwd), in the order of a saved forward-state row ([fp 3J |
+// R 9J | Jr 3J | GR 9J], pose_write_outputs): for J == BF_MAXJ the backward fetches the row with ONE bulk copy.  No tail
+// padding: PoseSmemBwd packs its scratch right behind it (see the size check there).
+struct PoseSmem {
+    float th[BF_THETA_SMEM];
     float sh[BF_MAXNS];
     float fp[BF_MAXJ * 3];
     float R[BF_MAXJ * 9];
@@ -23,7 +26,8 @@ struct __align__(16) PoseSmem {
     float GR[BF_MAXJ * 9];
     float Gt[BF_MAXJ * 3];
 };
-static_assert((BF_MAXNP + BF_MAXNS) % 4 == 0, "PoseSmem::fp must be 16-byte aligned");
+static_assert((BF_THETA_SMEM + BF_MAXNS) % 4 == 0 && offsetof(PoseSmem, fp) % 16 == 0, "PoseSmem::fp must be 16-byte aligned");
+static_assert(BF_THETA_SMEM >= BF_MAXNP - 9 + BF_MAXNS, "PoseSmem::th must hold the longest face-parameter row");
 // Backward scratch.  Everything else the backward needs lives in forward slots that are dead by then (smaller footprint ->
 // six CTAs of four frames per SM): d(posed joints) and later d(rel) in f.Gt (the backward never reads the posed joints),
 // d(full pose) in f.fp (each lane overwrites exactly the three angles it has just consumed), the updated theta in f.th, and --
@@ -34,14 +38,17 @@ struct __align__(16) PoseSmemBwd {
     float dGR[BF_MAXJ * 9];
     uint64_t bar;                 // mbarrier of the forward-state bulk copy
 };
-static_assert(BF_MAXNP <= 128 && 128 + BF_MAXJ * 3 <= BF_MAXJ * 9, "gradient row / d(rest joints) must fit into PoseSmem::R");
+// 13 CTAs of the default two frames fit into an SM's 228 KB (+ 1 KB per CTA): 2 * 8464 + 1024 = 17952 bytes per CTA.  The
+// face-parameter theta storage (BF_THETA_SMEM) fits into what the 16-byte tail padding of PoseSmem used to take.
+static_assert(sizeof(PoseSmemBwd) <= 8464, "k_pose_bwd: 13 CTAs of 2 frames per SM need <= 8464 bytes per frame");
+static_assert(BF_THETA_SMEM <= 128 && 128 + BF_MAXJ * 3 <= BF_MAXJ * 9, "gradient row / d(rest joints) must fit into PoseSmem::R");
 
 // Fills S for frame b (all lanes of one warp participate).
 __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmem& S, int lane);
 
 __device__ __forceinline__ void pose_forward_warp(const BfModel& m, const float* __restrict__ theta_row,
                                                   PoseSmem& S, int lane) {
-    const int np = theta_layout(m.is_smplx, m.NB).np;
+    const int np = theta_layout(m).np;
     for (int i = lane; i < np; i += 32) S.th[i] = theta_row[i];
     __syncwarp();
     pose_forward_from_smem(m, S, lane);
@@ -49,7 +56,7 @@ __device__ __forceinline__ void pose_forward_warp(const BfModel& m, const float*
 
 // theta already in S.th
 __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmem& S, int lane) {
-    const ThetaLayout L = theta_layout(m.is_smplx, m.NB);
+    const ThetaLayout L = theta_layout(m);
     const int J = m.J;
     // full pose
     for (int i = lane; i < 3 * J; i += 32) {
@@ -57,7 +64,7 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
         if (i < 3) v = S.th[4 + i];
         else if (i < 3 + L.nbody) v = S.th[7 + (i - 3)];
         else if (m.is_smplx) {
-            if (i < 69) v = 0.f;                                    // jaw: not optimised, stays 0
+            if (i < 69) v = m.face ? S.th[L.off_jaw + (i - 66)] : 0.f;   // jaw: 0 unless the model carries face parameters
             else if (i < 72) v = S.th[L.off_leye + (i - 69)];
             else if (i < 75) v = S.th[L.off_reye + (i - 72)];
             else if (i < 120) {
@@ -72,7 +79,7 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
         }
         S.fp[i] = v + __ldg(m.pose_mean + i);
     }
-    for (int l = lane; l < m.NS; l += 32) S.sh[l] = (l < m.NB) ? S.th[L.off_betas + l] : 0.f;
+    for (int l = lane; l < m.NS; l += 32) S.sh[l] = (l < m.NB) ? S.th[L.off_betas + l] : m.face ? S.th[L.off_expr + (l - m.NB)] : 0.f;
     __syncwarp();
     // rotations and rest joints
     for (int j = lane; j < J; j += 32) {
@@ -93,6 +100,8 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
                 acc += a.x * sh[0]; acc += a.y * sh[1]; acc += a.z * sh[2]; acc += a.w * sh[3];
                 acc += q.x * sh[4]; acc += q.y * sh[5]; acc += q.z * sh[6]; acc += q.w * sh[7];
                 acc += r.x * sh[8]; acc += r.y * sh[9];
+                if (m.face)                            // expression columns after the betas, in the order of the scalar loop
+                    for (int l = 10; l < m.NS; ++l) acc += __ldg(jd + l) * S.sh[l];
                 S.Jr[j * 3 + c] = __ldg(m.Jt + j * 3 + c) + acc;
             }
         } else {
@@ -100,7 +109,9 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
             for (int c = 0; c < 3; ++c) {
                 float acc = 0.f;
                 const float* jd = m.Jd + (j * 3 + c) * m.NS;
-                for (int l = 0; l < m.NB; ++l) acc += __ldg(jd + l) * S.sh[l];     // sh[l] = 0 for l >= NB (expression)
+                // sh[l] = 0 for l >= NB (expression) unless the model carries face parameters
+                const int nl = m.face ? m.NS : m.NB;
+                for (int l = 0; l < nl; ++l) acc += __ldg(jd + l) * S.sh[l];
                 S.Jr[j * 3 + c] = __ldg(m.Jt + j * 3 + c) + acc;
             }
         }
@@ -220,7 +231,9 @@ __global__ void __launch_bounds__(128) k_pose_fwd(BfModel m, BfFrames f) {
 //             ranks' halo buffers and raise the flag of the next iteration's tick (bf_pack.cuh)
 struct AdamArgs { float step_ts, step_lr, bc2_sqrt, beta2, om_beta1, om_beta2, eps; };
 
-__global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int flags, AdamArgs ad) {
+// (128, 7): at most 72 registers, so that the default launch shape (2 warps per CTA) keeps 13 CTAs per SM, the shared-memory
+// bound; without the cap the face-parameter code paths let ptxas take 96 registers, which would cut it to 10
+__global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int flags, AdamArgs ad) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     PoseSmemBwd* all = reinterpret_cast<PoseSmemBwd*>(smem_raw);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -231,7 +244,7 @@ __global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int fla
     float* const drel = S.Gt;
     float* const dfp = S.fp;
     const int J = m.J;
-    const ThetaLayout L = theta_layout(m.is_smplx, m.NB);
+    const ThetaLayout L = theta_layout(m);
     // ---- everything this frame reads from HBM is requested up front: the saved forward state by bulk copy (TMA), the
     // loss kernel's dA / dJtr rows, the Adam moments and the GMM gradient into registers; nothing below waits on HBM again
     // (J == BF_MAXJ: the row is one contiguous block of PoseSmem; smaller skeletons take the plain loops below)
@@ -428,6 +441,31 @@ __global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int fla
             g[L.off_betas + lane] = dsh + ((acc + a1) + a2);
         }
     }
+    if (m.face) {
+        // expression coefficients: the same rest-joint + blend-row sum as the betas above, in a lane pass of its own (so that
+        // the betas' lanes and summation order do not depend on the flag); lanes (e, part), NE = NS - NB
+        const int ne = m.NS - m.NB;
+        if (ne > 0) {
+            const int e = lane % ne, part = lane / ne;
+            const int nparts = 3 * ne <= 32 ? 3 : 2 * ne <= 32 ? 2 : 1;
+            const int nq = 3 * J, per = (nq + nparts - 1) / nparts;
+            float acc = 0.f;
+            if (part < nparts) {
+                const int q1 = min(nq, (part + 1) * per);
+                for (int q = part * per; q < q1; ++q) acc += __ldg(m.Jd + q * m.NS + m.NB + e) * dJr_s[q];
+            }
+            const float a1s = __shfl_sync(0xffffffffu, acc, (lane + ne) & 31);
+            const float a2s = __shfl_sync(0xffffffffu, acc, (lane + 2 * ne) & 31);
+            const float a1 = nparts > 1 ? a1s : 0.f;
+            const float a2 = nparts > 2 ? a2s : 0.f;
+            if (lane < ne) {
+                float dsh = f.dpf[(size_t)b * m.Kp + m.P + m.NB + lane];
+                if (f.dpf2) dsh += f.dpf2[(size_t)b * m.Kp + m.P + m.NB + lane];
+                g[L.off_expr + lane] = dsh + ((acc + a1) + a2);
+            }
+        }
+        if (lane < 3) g[L.off_jaw + lane] = dfp[66 + lane];                 // jaw: full-pose entries 66..68
+    }
     for (int i = lane; i < 3 + L.nbody; i += 32) g[4 + i] = dfp[i];      // global_orient + body_pose
     if (m.is_smplx) {
         if (lane < 3) { g[L.off_leye + lane] = dfp[69 + lane]; g[L.off_reye + lane] = dfp[72 + lane]; }
@@ -477,7 +515,18 @@ __global__ void __launch_bounds__(128) k_pose_bwd(BfModel m, BfFrames f, int fla
             sq = be * be;
             g[L.off_betas + lane] += f.w_shape * f.w_shape * 2.0f * be;
         }
-        const float shape_l = f.w_shape * f.w_shape * warp_sum(sq);
+        float shape_l = f.w_shape * f.w_shape * warp_sum(sq);
+        if (m.face) {
+            // expression prior w_expr^2 sum psi^2 (this project's choice; the reference optimises no expression).  It is
+            // reported with the shape prior.  No jaw prior: the reference defines none, so the jaw is held by the data alone.
+            float eq = 0.f;
+            if (lane < m.NS - m.NB) {
+                const float ps = S.th[L.off_expr + lane];
+                eq = ps * ps;
+                g[L.off_expr + lane] += f.w_expr * f.w_expr * 2.0f * ps;
+            }
+            shape_l += f.w_expr * f.w_expr * warp_sum(eq);
+        }
         if (lane == 0 && f.loss_terms) {
             f.loss_terms[b * 4 + 0] = total;
             f.loss_terms[b * 4 + 1] = pose_l;

@@ -22,7 +22,8 @@ class FrameBuffers(object):
     else the active set).  Owns the ``BfFrames`` struct passed to the library."""
 
     def __init__(self, model: PreparedModel, B, full=False, Nv=0, need_backward=True, n_trace=0,
-                 imsize=512.0, constant_scale=K.CONSTANT_SCALE_NO_SCAN, ext=None, temporal_weight=0.0):
+                 imsize=512.0, constant_scale=K.CONSTANT_SCALE_NO_SCAN, ext=None, temporal_weight=0.0,
+                 expr_weight=K.EXPR_PRIOR_WEIGHT):
         _lib.require_device()
         self.model, self.B, self.full = model, int(B), bool(full)
         dev = model.device
@@ -102,6 +103,7 @@ class FrameBuffers(object):
         s.lr_ts, s.lr = K.LR_TRANSL_SCALE, K.LR_DEFAULT
         s.beta1, s.beta2, s.eps = K.ADAM_BETAS[0], K.ADAM_BETAS[1], K.ADAM_EPS
         s.w_temporal = float(temporal_weight)
+        s.w_expr = float(expr_weight)              # read by face-parameter models only
         self.struct = s
 
     def bind(self, name, tensor):
@@ -154,7 +156,7 @@ class FitSession(object):
 
     def __init__(self, model: PreparedModel, B, Nv, num_iters, imsize=512, return_vertices=True,
                  chunk=4096, trace=True, dense_every_iter=False, temporal_weight=0.0, halo_exchange=None, out=None,
-                 halo=None, graph=None, sort_frames=None):
+                 halo=None, graph=None, sort_frames=None, expr_weight=K.EXPR_PRIOR_WEIGHT):
         """``out`` (optional): externally owned result buffers for these B frames -- ``theta`` [B,NP], ``verts`` [B,V,3],
         ``joints`` [B,K_full,3], ``full_pose`` [B,3J] (contiguous row slices of a larger batch: ConcurrentFitSession).
         ``halo``: a sharding.HaloLink -- boundary rows of the temporal term travel by in-kernel NVLink stores (graph-capturable);
@@ -166,13 +168,14 @@ class FitSession(object):
         128-frame tile of the blend GEMMs holds few rows and touches ~16 of the 30 vertex blocks of the SMPL-X active set
         (BfFrames.blk_mask).  Frames are independent fits, so the order is free; inputs are gathered and results scattered back
         by the packing kernels, all result tensors stay in the caller's frame order.  Default: on for SMPL-X batches of more
-        than one tile without the temporal term (which couples neighbours); BODYFIT_SORT=0 turns it off."""
+        than one tile without the temporal term (which couples neighbours); BODYFIT_SORT=0 turns it off.
+        ``expr_weight``: weight of the expression prior of a face-parameter model (ignored otherwise)."""
         self.model, self.B, self.Nv, self.N = model, int(B), int(Nv), int(num_iters)
         assert self.N >= 1
         dev = model.device
         out = out or {}
         self.fb = FrameBuffers(model, B, full=False, Nv=Nv, n_trace=(self.N if trace else 0), imsize=imsize,
-                               temporal_weight=temporal_weight)
+                               temporal_weight=temporal_weight, expr_weight=expr_weight)
         if sort_frames is None:
             sort_frames = os.environ.get('BODYFIT_SORT', '1') != '0'
         self.sort_frames = bool(sort_frames) and model.is_smplx and temporal_weight <= 0 and self.B > 128 and 'blk_mask' in self.fb.t
@@ -442,6 +445,8 @@ class FitSession(object):
         if m.is_smplx:
             out.update(leye_pose=sn['leye_pose'], reye_pose=sn['reye_pose'],
                        left_hand_pose=sn['left_hand_pose'], right_hand_pose=sn['right_hand_pose'])
+        if m.face_params:
+            out.update(jaw_pose=sn['jaw_pose'], expression=sn['expression'])
         return out
 
 
@@ -483,7 +488,8 @@ class ConcurrentFitSession(object):
     Same interface as FitSession (set_inputs / run / results)."""
 
     def __init__(self, model: PreparedModel, B, Nv, num_iters, imsize=512, return_vertices=True, dense_every_iter=False,
-                 n_parts=4, trace=True, min_part=2048, lead=0, taper=0.5, graph=None, sort_frames=None):
+                 n_parts=4, trace=True, min_part=2048, lead=0, taper=0.5, graph=None, sort_frames=None,
+                 expr_weight=K.EXPR_PRIOR_WEIGHT):
         self.model, self.B, self.Nv, self.N = model, int(B), int(Nv), int(num_iters)
         dev = model.device
         self.ranges = staggered_ranges(self.B, n_parts, min_part=min_part, lead=lead, taper=taper)
@@ -501,7 +507,8 @@ class ConcurrentFitSession(object):
             out = dict(theta=self.theta[lo:hi], joints=self.joints[lo:hi], full_pose=self.full_pose[lo:hi],
                        verts=self.verts[lo:hi] if return_vertices else None)
             self.parts.append(FitSession(model, hi - lo, Nv, num_iters, imsize=imsize, return_vertices=return_vertices,
-                                         dense_every_iter=dense_every_iter, trace=trace, out=out, graph=graph, sort_frames=sort_frames))
+                                         dense_every_iter=dense_every_iter, trace=trace, out=out, graph=graph, sort_frames=sort_frames,
+                                         expr_weight=expr_weight))
             self.streams.append(torch.cuda.Stream(device=dev))
             self.prio_streams.append(torch.cuda.Stream(device=dev, priority=min(lowest, max(highest, highest + k))))
         self.kernel_launches = 0
@@ -550,4 +557,6 @@ class ConcurrentFitSession(object):
         if m.is_smplx:
             out.update(leye_pose=sn['leye_pose'], reye_pose=sn['reye_pose'],
                        left_hand_pose=sn['left_hand_pose'], right_hand_pose=sn['right_hand_pose'])
+        if m.face_params:
+            out.update(jaw_pose=sn['jaw_pose'], expression=sn['expression'])
         return out

@@ -32,7 +32,7 @@ from . import constants as K
 
 
 MAX_NS = 20         # betas + expression coefficients per frame (BF_MAXNS, csrc/bf_common.cuh)
-MAX_NP = 100        # theta entries per frame (BF_MAXNP)
+MAX_NP = 100        # theta entries per frame without the face block (BF_MAXNP)
 
 
 def _round_up(x, m):
@@ -76,7 +76,7 @@ def load_model_data(path_or_dict, model_type=None, gender='neutral'):
 
 
 def model_desc(smpl_type, data, gmm=None, J_regressor_extra=None, num_betas=10, num_expression=10, tensor_cores=True,
-               gender='neutral', kid_template=None):
+               gender='neutral', kid_template=None, face_params=False):
     """``(BfModelDesc, keepalive)`` for ``bf_model_create`` / ``bf_model_build_blob``: the raw model arrays as the C ABI
     takes them (what a non-Python host would pass after reading the model file itself)."""
     data = load_model_data(data, smpl_type, gender)
@@ -99,6 +99,7 @@ def model_desc(smpl_type, data, gmm=None, J_regressor_extra=None, num_betas=10, 
     d.parents, d.faces = arr(np.asarray(data['kintree_table'])[0].astype(np.int64), np.int32), arr(faces, np.int32)
     d.is_smplx, d.V, d.J, d.F, d.n_shape_dirs = int(smpl_type == 'smplx'), vt.shape[0], W.shape[1], faces.shape[0], sd.shape[2]
     d.num_betas, d.num_expression, d.tensor_cores = num_betas, num_expression, int(bool(tensor_cores))
+    d.face_params = int(bool(face_params))
     if smpl_type == 'smplx':
         d.hands_meanl, d.hands_meanr = arr(data['hands_meanl'], np.float32), arr(data['hands_meanr'], np.float32)
         d.hands_componentsl, d.hands_componentsr = arr(data['hands_componentsl'], np.float32), arr(data['hands_componentsr'], np.float32)
@@ -119,10 +120,13 @@ def model_desc(smpl_type, data, gmm=None, J_regressor_extra=None, num_betas=10, 
 
 
 class PreparedModel(object):
-    """numpy tables -> device tensors -> BfModel struct (kept alive by this object)."""
+    """numpy tables -> device tensors -> BfModel struct (kept alive by this object).
+
+    ``face_params=True`` (SMPL-X only) builds a face-parameter model: theta rows end with [jaw 3 | expression NE], which the
+    operator takes as inputs and the fit optimises.  Without it the jaw and the expression stay at zero, as in the reference."""
 
     def __init__(self, smpl_type, data, gmm=None, J_regressor_extra=None, device='cuda', num_betas=10,
-                 num_expression=10, tensor_cores=None, gender='neutral', age='adult', kid_template=None):
+                 num_expression=10, tensor_cores=None, gender='neutral', age='adult', kid_template=None, face_params=False):
         assert smpl_type in ('smpl', 'smplx')
         self.smpl_type = smpl_type
         self.is_smplx = smpl_type == 'smplx'
@@ -143,6 +147,9 @@ class PreparedModel(object):
         P = (J - 1) * 9
         if num_betas < 1 or (self.is_smplx and num_expression < 0):
             raise ValueError('num_betas must be at least 1 and num_expression not negative')
+        if face_params and not self.is_smplx:
+            raise ValueError('face parameters (jaw pose, expression) apply to SMPL-X only')
+        self.face_params = bool(face_params)
         NB = num_betas
         sd_all = np.asarray(data['shapedirs'], dtype=np.float32)
         if sd_all.ndim == 2:
@@ -173,6 +180,9 @@ class PreparedModel(object):
             raise ValueError('%d shape coefficients (betas + expression) exceed the limit of %d' % (NS, MAX_NS))
         if NP > MAX_NP:
             raise ValueError('%d theta entries exceed the limit of %d' % (NP, MAX_NP))
+        self.NE = NS - NB
+        if self.face_params:
+            NP += 3 + self.NE                       # [jaw 3 | expression NE]; bounded by MAX_NS, at most 111 entries
         if self.is_smplx and sd_all.shape[-1] >= K.SHAPE_SPACE_DIM + num_expression:
             # official files: the expression directions follow the 300 shape directions (smplx: SHAPE_SPACE_DIM)
             sd = np.concatenate([sd_all[:, :, :NB], sd_all[:, :, K.SHAPE_SPACE_DIM:K.SHAPE_SPACE_DIM + num_expression]], -1)
@@ -316,7 +326,7 @@ class PreparedModel(object):
         self._fill_vset(self.struct.full, 'full', full_h)
         self._fill_vset(self.struct.act, 'act', act_h)
         for k, v in dict(J=J, P=P, NS=NS, NB=NB, Kp=self.Kp, NP=self.NP, is_smplx=int(self.is_smplx),
-                         max_depth=self.max_depth, K_used=K_used, n_gmm=self.n_gmm).items():
+                         max_depth=self.max_depth, K_used=K_used, n_gmm=self.n_gmm, face=int(self.face_params)).items():
             setattr(self.struct, k, v)
         self.n_act = int(act_h['n'])
         self.n_pad_full = int(full_h['n_pad'])
@@ -539,8 +549,9 @@ class PreparedModel(object):
         return path
 
     def pack_theta(self, global_orient, body_pose, betas, transl=None, scale=None, leye=None, reye=None,
-                   lhand=None, rhand=None):
-        """Assemble [B, NP] theta rows (layout in include/bodyfit_b200.h)."""
+                   lhand=None, rhand=None, jaw=None, expression=None):
+        """Assemble [B, NP] theta rows (layout in include/bodyfit_b200.h).  ``jaw`` [B,3] / ``expression`` [B,NE] belong to a
+        face-parameter model (None = 0); a face-off model accepts them only as None."""
         B = global_orient.shape[0]
         dev, dt = self.device, torch.float32
         z = lambda n: torch.zeros(B, n, device=dev, dtype=dt)
@@ -552,6 +563,10 @@ class PreparedModel(object):
                  f(global_orient, 3), f(body_pose, self.nbody), bt]
         if self.is_smplx:
             parts += [f(leye, 3), f(reye, 3), f(lhand, 6), f(rhand, 6)]
+        if self.face_params:
+            parts += [f(jaw, 3), f(expression, self.NE)]
+        elif jaw is not None or expression is not None:
+            raise ValueError('jaw / expression need a face-parameter SMPL-X model (face_params=True)')
         return torch.cat(parts, dim=1).contiguous()
 
     def split_theta(self, theta):
@@ -562,4 +577,6 @@ class PreparedModel(object):
             o = 7 + nb + self.NB
             out.update(leye_pose=theta[:, o:o + 3], reye_pose=theta[:, o + 3:o + 6],
                        left_hand_pose=theta[:, o + 6:o + 12], right_hand_pose=theta[:, o + 12:o + 18])
+            if self.face_params:
+                out.update(jaw_pose=theta[:, o + 18:o + 21], expression=theta[:, o + 21:o + 21 + self.NE])
         return out

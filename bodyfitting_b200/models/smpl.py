@@ -79,28 +79,30 @@ class SMPL(nn.Module):
 
 
 class SMPLX(nn.Module):
-    """SMPL-X as ``SMPLify.__init__`` builds it: 6 PCA hand components, 10 betas + 10 (zero) expression
-    coefficients, contour landmarks, joints mapped to the 135 OpenPose keypoints (smplify.py:59-80)."""
+    """SMPL-X as ``SMPLify.__init__`` builds it: 6 PCA hand components, 10 betas + 10 expression coefficients, contour
+    landmarks, joints mapped to the 135 OpenPose keypoints (smplify.py:59-80).  Built as a face-parameter model, so
+    ``forward`` takes ``jaw_pose`` and ``expression`` like ``smplx.SMPLX.forward``, with gradients (None = 0)."""
 
-    def __init__(self, model_data, device='cuda', **kwargs):
+    def __init__(self, model_data, device='cuda', num_betas=10, num_expression=10, **kwargs):
         super().__init__()
-        self.prepared = PreparedModel('smplx', model_data, gmm=None, device=device)
+        self.prepared = PreparedModel('smplx', model_data, gmm=None, device=device, num_betas=num_betas,
+                                      num_expression=num_expression, face_params=True)
         self.faces = self.prepared.faces
 
     def forward(self, global_orient=None, body_pose=None, betas=None, jaw_pose=None, leye_pose=None, reye_pose=None,
-                left_hand_pose=None, right_hand_pose=None, return_full_pose=False, **kwargs):
+                left_hand_pose=None, right_hand_pose=None, expression=None, return_full_pose=False, **kwargs):
+        """``jaw_pose`` [B,3] or [B,1,3], ``expression`` [B,NE]; both differentiable, None = 0."""
         pm = self.prepared
-        if jaw_pose is not None and bool((jaw_pose != 0).any()):
-            raise NotImplementedError('jaw_pose is held at zero on this path (not optimised by the reference, smplify.py:118,167-173)')
         theta = pm.pack_theta(global_orient, body_pose, betas, leye=leye_pose, reye=reye_pose, lhand=left_hand_pose,
-                              rhand=right_hand_pose)
+                              rhand=right_hand_pose, jaw=jaw_pose, expression=expression)
         verts, joints, full_pose = ops.lbs(theta, pm)
-        return ModelOutput(vertices=verts, joints=joints, betas=betas, global_orient=global_orient, body_pose=body_pose,
-                           left_hand_pose=left_hand_pose, right_hand_pose=right_hand_pose, jaw_pose=jaw_pose,
-                           full_pose=full_pose if return_full_pose else None)
+        return ModelOutput(vertices=verts, joints=joints, betas=betas, expression=expression, global_orient=global_orient,
+                           body_pose=body_pose, left_hand_pose=left_hand_pose, right_hand_pose=right_hand_pose,
+                           jaw_pose=jaw_pose, full_pose=full_pose if return_full_pose else None)
 
 
-def create_smplx(model_path='data', gender='neutral', model_data=None, device='cuda', **kwargs):
+def create_smplx(model_path='data', gender='neutral', model_data=None, device='cuda', num_betas=10, num_expression=10,
+                 **kwargs):
     from ..model import load_model_data
     data = model_data if model_data is not None else load_model_data(model_path, 'smplx', gender)
-    return SMPLX(data, device=device)
+    return SMPLX(data, device=device, num_betas=num_betas, num_expression=num_expression)

@@ -18,7 +18,9 @@ from .smplify import SMPLify
 
 class BodyFitting(object):
     def __init__(self, options=None, smpl_type=None, age='adult', use_mask=False, debug=False, init_fn=None, regressor=None,
-                 **smplify_kw):
+                 face_params=False, **smplify_kw):
+        """``face_params=True`` (SMPL-X): the fits also optimise jaw pose and expression (SMPLify(face_params=)); the results
+        and the saved parameter file then hold ``jaw_pose`` and ``expression``."""
         self.options = options
         self.smpl_type = smpl_type or getattr(options, 'smpl_type', 'smpl')
         self.age = getattr(options, 'age', age)
@@ -27,6 +29,7 @@ class BodyFitting(object):
         self.use_hand_face = (self.smpl_type == 'smplx')
         self.init_fn = init_fn
         self.regressor = regressor
+        self.face_params = bool(getattr(options, 'face_params', face_params))
         self.smplify_kw = smplify_kw
         self._smplify = {}
 
@@ -37,7 +40,7 @@ class BodyFitting(object):
             if num_iters is not None:
                 kw['num_iters'] = num_iters
             self._smplify[key] = SMPLify(smpl_type=self.smpl_type, age=self.age, gender=gender, use_mask=self.use_mask,
-                                         debug=False, **kw)
+                                         debug=False, face_params=self.face_params, **kw)
         return self._smplify[key]
 
     def __call__(self, images, c2ws, Ks, keypoints, gender='male', keyframe=25, use_frames=list(range(48)),
@@ -64,7 +67,8 @@ class BodyFitting(object):
 
 
 def write_result(output_folder, smpl_type, result, disp=False):
-    """``{smpl_type}_parameter.npy`` (pickled dict) + ``{smpl_type}.obj`` (+ ``{smpl_type}+d.obj``), body_fitting.py:94-99"""
+    """``{smpl_type}_parameter.npy`` (pickled dict) + ``{smpl_type}.obj`` (+ ``{smpl_type}+d.obj``), body_fitting.py:94-99.
+    The parameter file holds every key of ``result``: ``jaw_pose`` / ``expression`` too when the fit optimised them."""
     os.makedirs(output_folder, exist_ok=True)
     np.save(os.path.join(output_folder, '%s_parameter.npy' % smpl_type), result)
     save_obj_mesh(os.path.join(output_folder, '%s.obj' % smpl_type), result['vertices'], result['faces'])

@@ -35,11 +35,18 @@ class SMPLify(object):
                  gender='male', use_mask=False, device=torch.device('cuda'), debug=True,
                  model_data=None, gmm=None, J_regressor_extra=None, data_root='data', dense_every_iter=False,
                  concurrent_parts=None, concurrent_min_part=512, temporal_weight=0.0, halo_exchange=None, halo=None,
-                 copy_outputs=None, graph=None, sort_frames=None, kid_template=None):
+                 copy_outputs=None, graph=None, sort_frames=None, kid_template=None, face_params=False,
+                 expr_prior_weight=K.EXPR_PRIOR_WEIGHT):
+        """``face_params=True`` (SMPL-X only): the fit also optimises the jaw pose and the expression coefficients, with the
+        expression prior ``expr_prior_weight^2 * sum psi^2`` (the reference optimises neither, smplify.py:118,167-173; no jaw
+        prior).  The result dict then also holds ``jaw_pose`` and ``expression``."""
         if age not in ('adult', 'kid'):
             raise ValueError("age must be 'adult' or 'kid' (smplify.py:23,112-115)")
         if age == 'kid' and smpl_type != 'smpl':
             raise ValueError("age='kid' exists for smpl_type='smpl' only: the reference passes it to the SMPL branch (smplify.py:50-56)")
+        if face_params and smpl_type != 'smplx':
+            raise ValueError("face_params=True needs smpl_type='smplx': SMPL has no jaw / expression parameters")
+        self.face_params, self.expr_prior_weight = bool(face_params), float(expr_prior_weight)
         self.device = torch.device(device)
         self.debug = debug
         self.gender = gender
@@ -63,7 +70,8 @@ class SMPLify(object):
         if age == 'kid' and kid_template is None:
             kid_template = os.path.join(data_root, 'smil', 'smil_web.pkl')           # config.SMIL_MODEL_DIR (config.py:5)
         self.model = PreparedModel(smpl_type, model_data, gmm=gmm, J_regressor_extra=J_regressor_extra,
-                                   device=self.device, gender=gender, age=age, kid_template=kid_template)
+                                   device=self.device, gender=gender, age=age, kid_template=kid_template,
+                                   face_params=self.face_params)
         self.smpl_faces = self.model.faces.astype(np.int32).reshape(1, -1, 3)
         self.last_trace = None
         self.dense_every_iter = dense_every_iter
@@ -234,7 +242,8 @@ class SMPLify(object):
             scan_height = float((scan_verts.max(0) - scan_verts.min(0))[1])
             constant_scale = scan_height / 1.7                                            # smplify.py:156
             searcher = MeshGridSearcher(verts=scan_verts, faces=scan_faces, device=dev)
-        fb = FrameBuffers(m, B, full=True, Nv=Nv, n_trace=N, imsize=imsize, constant_scale=constant_scale)
+        fb = FrameBuffers(m, B, full=True, Nv=Nv, n_trace=N, imsize=imsize, constant_scale=constant_scale,
+                          expr_weight=self.expr_prior_weight)
         kp_dev = self._h2d('kp', kp)
         poses_dev, betas_dev = self._h2d('poses', init_poses), self._h2d('betas', init_betas)
         fb.bind('kp', pack_keypoints(kp_dev, self.use_hand_face))
@@ -280,6 +289,8 @@ class SMPLify(object):
         if m.is_smplx:
             out.update(leye_pose=sn['leye_pose'], reye_pose=sn['reye_pose'],
                        left_hand_pose=sn['left_hand_pose'], right_hand_pose=sn['right_hand_pose'])
+        if m.face_params:
+            out.update(jaw_pose=sn['jaw_pose'], expression=sn['expression'])
         self.last_trace, self.last_loss_terms = fb.t['trace'], fb.t['loss_terms']
         self.last_pc_loss = pc if use_mesh else None
         self.last_mask_loss = sil.mask_loss if sil is not None else None
@@ -327,11 +338,13 @@ class SMPLify(object):
                 cache[key] = ConcurrentFitSession(self.model, B, Nv, self.num_iters, imsize=imsize, return_vertices=return_vertices,
                                                   dense_every_iter=self.dense_every_iter, n_parts=n_parts,
                                                   min_part=min_part, lead=self.concurrent_lead,
-                                                  taper=self.concurrent_taper, graph=self.graph, sort_frames=self.sort_frames)
+                                                  taper=self.concurrent_taper, graph=self.graph, sort_frames=self.sort_frames,
+                                                  expr_weight=self.expr_prior_weight)
             else:
                 cache[key] = FitSession(self.model, B, Nv, self.num_iters, imsize=imsize,
                                         return_vertices=return_vertices, dense_every_iter=self.dense_every_iter,
                                         temporal_weight=self.temporal_weight, halo_exchange=self.halo_exchange, halo=self.halo,
+                                        expr_weight=self.expr_prior_weight,
                                         graph=self.graph, sort_frames=self.sort_frames)
         cache[('last', base)] = bool(host_io)
         return cache[key]

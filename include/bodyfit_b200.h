@@ -24,7 +24,10 @@
  * All floating point data is fp32, row-major, contiguous unless a leading dimension
  * is given.  "theta" is the per-frame optimisation vector:
  *   [transl 3 | scale 1 | global_orient 3 | body_pose 69(smpl) or 63(smplx) | betas 10 |
- *    (smplx only) leye 3 | reye 3 | left_hand_pca 6 | right_hand_pca 6]      NP = 86 / 98
+ *    (smplx only) leye 3 | reye 3 | left_hand_pca 6 | right_hand_pca 6 |
+ *    (face-parameter smplx model only, BfModel.face) jaw 3 | expression NE]   NP = 86 / 98 / 98 + 3 + NE
+ * with 10 betas (num_betas in general; 11 for the kid model).  The face block of a face-parameter model
+ * (BfModelDesc.face_params) follows every other entry, so all other offsets are the same with and without it.
  */
 #ifndef BODYFIT_B200_H
 #define BODYFIT_B200_H
@@ -40,7 +43,7 @@ extern "C" {
 #define BF_ECUDA    -2   /* a CUDA runtime call / launch failed            */
 #define BF_EARCH    -3   /* device is not sm_100 (no fallback exists)      */
 
-#define BF_ABI_VERSION 19
+#define BF_ABI_VERSION 20
 #define BF_F_WORLD 1   /* forward outputs in world space: (x + transl) * scale * constant_scale */
 #define BF_F_TC    2   /* run the blend-shape contractions on tcgen05 tensor cores (3xTF32) */
 #define BF_F_SKIN_FUSED 4  /* bf_frame_loss_backward skins the frame's live vertices itself from vposed (after bf_blend_forward) */
@@ -106,7 +109,9 @@ typedef struct BfModel {
     const float*   gmm_bt_lo;
     BfVSet full;
     BfVSet act;
-    int32_t J, P, NS, NB, Kp, NP, is_smplx, max_depth, K_used, n_gmm, _pad0, _pad1;
+    int32_t J, P, NS, NB, Kp, NP, is_smplx, max_depth, K_used, n_gmm;
+    int32_t face;             /* 1 = face-parameter SMPL-X model: theta carries jaw pose + the NS - NB expression coefficients */
+    int32_t _pad1;
 } BfModel;
 
 /* Per-call frame buffers (all device memory, B frames). */
@@ -132,7 +137,7 @@ typedef struct BfFrames {
     const float* kp;         /* [B,K_used,Nv,3] (x, y, effective weight), joint-major: the views of a joint are contiguous */
     const float* cams;       /* [Nv,12] row-major 3x4  K @ [R|t] (world -> pixel, homogeneous) */
     float*       loss;       /* [B] per-frame total loss of this iteration */
-    float*       loss_terms; /* [B,4] data, pose prior, angle prior, shape prior (optional) */
+    float*       loss_terms; /* [B,4] data, pose prior, angle prior, shape prior (+ expression prior, face models) (optional) */
     float*       trace;      /* [n_iters,B] optional per-iteration loss trace */
     float*       pf_hi;      /* [B,Kp]  3xTF32 split of pf (BF_F_TC) */
     float*       pf_lo;
@@ -166,7 +171,9 @@ typedef struct BfFrames {
     int32_t flags;             /* BF_F_WORLD: skin/joints forward write (x + transl) * scale * constant_scale (smplify.py:189-190) */
     int32_t halo_iters;        /* NVLink halo: iterations of the run; iteration `iter` publishes its updated boundary rows iff iter + 1 < halo_iters */
     float imsize, constant_scale, sigma, w_pose, w_angle, w_shape;
-    float w_temporal, _padf;   /* weight of the temporal term (0 = off; not part of the reference) */
+    float w_temporal;          /* weight of the temporal term (0 = off; not part of the reference) */
+    float w_expr;              /* face models: expression prior w_expr^2 sum psi^2 (this project's term, the reference has none;
+                                  bf_frames_bind sets 5).  Face-off models ignore it.  There is no jaw prior. */
 } BfFrames;
 
 int         bf_abi_version(void);
@@ -256,9 +263,11 @@ typedef struct BfModelDesc {
     const float*   gmm_covars;              /* [n_gmm,69,69] */
     const float*   gmm_weights;             /* [n_gmm] */
     /* num_betas >= 1 (the kid template adds one more); num_expression >= 0 (SMPL-X only; 0 = no expression directions).
-     * The model is rejected when betas + expression exceed 20 or its theta row exceeds 100 entries (NP above). */
+     * The model is rejected when betas + expression exceed 20 or its theta row without the face block exceeds 100 entries
+     * (NP above).  face_params != 0 (SMPL-X only): theta also carries the jaw pose and the expression coefficients, which the
+     * fit then optimises (at most 91 + 20 = 111 entries); 0 keeps them at zero, as the reference does. */
     int32_t is_smplx, V, J, F, n_shape_dirs, num_betas, num_expression, n_lmk, n_dyn_rows, n_dyn, n_extra_vids, n_regressor_extra,
-            n_gmm, tensor_cores, _pad0, _pad1;
+            n_gmm, tensor_cores, face_params, _pad1;
 } BfModelDesc;
 int     bf_model_create(const BfModelDesc* desc, BfModel** out);
 int     bf_model_build_blob(const BfModelDesc* desc, void** blob, int64_t* nbytes);
