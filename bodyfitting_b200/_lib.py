@@ -10,7 +10,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('BODYFIT_LIB') or os.path.join(_HERE, 'libbodyfit_b200.so')   # BODYFIT_LIB: A/B builds of the same ABI
-ABI_VERSION = 20
+ABI_VERSION = 21
 F_WORLD = 1
 F_TC = 2
 F_SKIN_FUSED = 4
@@ -34,7 +34,8 @@ class BfModelDesc(C.Structure):
         'hands_componentsl', 'hands_componentsr', 'lmk_faces_idx', 'lmk_bary_coords', 'dynamic_lmk_faces_idx',
         'dynamic_lmk_bary_coords', 'extra_vids', 'J_regressor_extra', 'kid_template', 'gmm_means', 'gmm_covars', 'gmm_weights')] + \
         [(n, _i32) for n in ('is_smplx', 'V', 'J', 'F', 'n_shape_dirs', 'num_betas', 'num_expression', 'n_lmk', 'n_dyn_rows', 'n_dyn',
-                             'n_extra_vids', 'n_regressor_extra', 'n_gmm', 'tensor_cores', 'face_params', '_pad1')]
+                             'n_extra_vids', 'n_regressor_extra', 'n_gmm', 'tensor_cores', 'face_params', 'num_pca_comps')] + \
+        [(n, C.c_uint32) for n in ('hand_axis_angle', 'flat_hand_mean')]
 
 
 class BfModel(C.Structure):
@@ -43,7 +44,7 @@ class BfModel(C.Structure):
         'gmm_mean', 'gmm_psym', 'gmm_logw', 'gmm_bt_hi', 'gmm_bt_lo')] + \
         [('full', BfVSet), ('act', BfVSet)] + \
         [(n, _i32) for n in ('J', 'P', 'NS', 'NB', 'Kp', 'NP', 'is_smplx', 'max_depth', 'K_used',
-                             'n_gmm', 'face', '_pad1')]
+                             'n_gmm', 'face', 'n_hand')]
 
 
 class BfFrames(C.Structure):

@@ -35,7 +35,8 @@ static int check_model(const BfModel* m, const BfFrames* f) {
     BF_REQUIRE(m->J > 0 && m->J <= BF_MAXJ, "J out of range");
     BF_REQUIRE(m->NS > 0 && m->NS <= BF_MAXNS && m->NB <= m->NS, "NS/NB out of range");
     BF_REQUIRE(m->face == 0 || (m->face == 1 && m->is_smplx), "face parameters apply to SMPL-X only");
-    BF_REQUIRE(m->NP == theta_layout(*m).np && theta_layout(m->is_smplx, m->NB).np <= BF_MAXNP && m->NP <= BF_THETA_SMEM,
+    BF_REQUIRE(!m->is_smplx || (m->n_hand >= 1 && m->n_hand <= BF_MAXHAND), "n_hand out of range");
+    BF_REQUIRE(m->NP == theta_layout(*m).np && theta_layout(m->is_smplx, m->NB).np <= BF_MAXNP && m->NP <= BF_THETA_SMEM_WIDE,
                "NP does not match theta layout");
     BF_REQUIRE(m->Kp % 16 == 0 && m->Kp >= m->P + m->NS + 1, "Kp must be a multiple of 16 covering P+NS+1");
     BF_REQUIRE(m->P == (m->J - 1) * 9, "P != 9(J-1)");
@@ -89,7 +90,10 @@ int bf_pose_forward(const BfModel* m, const BfFrames* f, void* stream) {
     BF_REQUIRE(f->pf && f->A && f->Jtr, "pf/A/Jtr is null");
     const int wpb = 4;
     const dim3 grid((f->B + wpb - 1) / wpb), block(32 * wpb);
-    k_pose_fwd<<<grid, block, wpb * sizeof(PoseSmem), (cudaStream_t)stream>>>(*m, *f);
+    if (m->NP <= BF_THETA_SMEM)                             // every row of at most 112 entries
+        k_pose_fwd<BF_THETA_SMEM><<<grid, block, wpb * sizeof(PoseSmem), (cudaStream_t)stream>>>(*m, *f);
+    else
+        k_pose_fwd<BF_THETA_SMEM_WIDE><<<grid, block, wpb * sizeof(PoseSmemWide), (cudaStream_t)stream>>>(*m, *f);
     BF_LAUNCH_CHECK();
     return BF_OK;
 }
@@ -400,7 +404,10 @@ int bf_pose_backward(const BfModel* m, const BfFrames* f, int flags, void* strea
     const dim3 grid((f->B + wpb - 1) / wpb), block(32 * wpb);
     BfFrames g = *f;
     if (!bf_bwd_two_cta(m, f)) g.dpf2 = nullptr;         // the backward GEMM added its two half-reductions itself
-    k_pose_bwd<<<grid, block, wpb * sizeof(PoseSmemBwd), (cudaStream_t)stream>>>(*m, g, flags, ad);
+    if (m->NP <= BF_THETA_SMEM)
+        k_pose_bwd<BF_THETA_SMEM><<<grid, block, wpb * sizeof(PoseSmemBwd), (cudaStream_t)stream>>>(*m, g, flags, ad);
+    else
+        k_pose_bwd<BF_THETA_SMEM_WIDE><<<grid, block, wpb * sizeof(PoseSmemBwdWide), (cudaStream_t)stream>>>(*m, g, flags, ad);
     BF_LAUNCH_CHECK();
     return BF_OK;
 }

@@ -9,8 +9,10 @@
 
 #define BF_MAXJ 55          // SMPL-X kinematic tree
 #define BF_MAXNS 20         // 10 betas + 10 expression coefficients
-#define BF_MAXNP 100        // theta entries without the face block (86 / 98)
-#define BF_THETA_SMEM 112   // per-frame theta storage: a face-parameter row adds 3 + NE <= 23 entries (at most 111)
+#define BF_MAXNP 100        // theta entries without the face block, counted with 6 hand components (86 / 98)
+#define BF_THETA_SMEM 112   // per-frame theta storage of the pose kernels: a face-parameter row adds 3 + NE <= 23 entries (at most 111)
+#define BF_THETA_SMEM_WIDE 192   // ... of their wide instantiation, for rows longer than 112 (wider hands: at most 189 entries)
+#define BF_MAXHAND 45       // hand parameters per hand: PCA components, or the 45 axis-angle entries
 #define BF_GMM_D 69
 
 void bf_set_error(const char* fmt, ...);
@@ -70,21 +72,22 @@ struct ThetaLayout {
 };
 // nbetas: 10, or 11 for the SMPL kid model (age='kid': the SMIL template difference is an extra shape direction)
 // face (SMPL-X only): the row ends with [jaw 3 | expression nexpr]; without it off_jaw = off_expr = np
-__host__ __device__ __forceinline__ ThetaLayout theta_layout(int is_smplx, int nbetas = 10, int face = 0, int nexpr = 0) {
+// nhand (SMPL-X only): hand parameters per hand (PCA components, or 45 axis-angle entries)
+__host__ __device__ __forceinline__ ThetaLayout theta_layout(int is_smplx, int nbetas = 10, int face = 0, int nexpr = 0, int nhand = 6) {
     ThetaLayout t;
     t.nbody = is_smplx ? 63 : 69;
     t.off_betas = 7 + t.nbody;
     t.off_leye = t.off_betas + nbetas;
     t.off_reye = t.off_leye + 3;
     t.off_lh = t.off_reye + 3;
-    t.off_rh = t.off_lh + 6;
-    t.off_jaw = is_smplx ? t.off_rh + 6 : t.off_betas + nbetas;
+    t.off_rh = t.off_lh + nhand;
+    t.off_jaw = is_smplx ? t.off_rh + nhand : t.off_betas + nbetas;
     t.off_expr = t.off_jaw + ((is_smplx && face) ? 3 : 0);
     t.np = t.off_expr + ((is_smplx && face) ? nexpr : 0);
     return t;
 }
 __host__ __device__ __forceinline__ ThetaLayout theta_layout(const BfModel& m) {
-    return theta_layout(m.is_smplx, m.NB, m.face, m.NS - m.NB);
+    return theta_layout(m.is_smplx, m.NB, m.face, m.NS - m.NB, m.n_hand);
 }
 
 // round-to-nearest TF32 (10-bit mantissa, low 13 bits zero) and the exact fp32 remainder: x = hi + lo

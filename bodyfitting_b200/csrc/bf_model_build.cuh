@@ -340,6 +340,13 @@ struct Builder {
         if (NB < 1 || NE < 0) { err = "num_betas must be at least 1 and num_expression not negative"; return false; }
         if (d.face_params && !smplx) { err = "face parameters (jaw pose, expression) apply to SMPL-X only"; return false; }
         const bool face = smplx && d.face_params != 0;
+        // hand options (smplx.create's num_pca_comps / use_pca / flat_hand_mean); num_pca_comps 0 means 6
+        const int npca = d.num_pca_comps == 0 ? 6 : d.num_pca_comps;
+        if (!smplx && (npca != 6 || d.hand_axis_angle || d.flat_hand_mean)) {
+            err = "hand options (num_pca_comps, use_pca, flat_hand_mean) apply to SMPL-X only"; return false;
+        }
+        if (npca < 1 || npca > 45) { err = "num_pca_comps must be between 1 and 45"; return false; }
+        const int nhand = !smplx ? 0 : d.hand_axis_angle ? 45 : npca;
         const int S = d.n_shape_dirs;
         vt.assign(d.v_template, d.v_template + (size_t)V * 3);
         // shape directions: [V,3,NB] (+ the kid direction) (+ NE expression directions; official files keep them after 300)
@@ -376,7 +383,8 @@ struct Builder {
         // the face block; that block (3 + NE entries) is bounded by the shape limit, so a face row has at most 111 entries.
         if (NS > BF_MAXNS) { snprintf(msg, sizeof(msg), "%d shape coefficients (betas + expression) exceed the limit of %d", NS, BF_MAXNS); err = msg; return false; }
         if (NP > BF_MAXNP) { snprintf(msg, sizeof(msg), "%d theta entries exceed the limit of %d", NP, BF_MAXNP); err = msg; return false; }
-        if (face) NP += 3 + NE;                          // [jaw 3 | expression NE] after the right-hand PCA
+        if (smplx) NP += 2 * (nhand - 6);                // the 100-entry limit counts 6 hand parameters; at most 189 entries
+        if (face) NP += 3 + NE;                          // [jaw 3 | expression NE] after the right-hand parameters
 
         // kinematic tree
         std::vector<int32_t> parents(J), depth(J, 0), child_ptr(J + 1, 0), child_idx;
@@ -414,9 +422,16 @@ struct Builder {
         std::vector<float> pose_mean(3 * J, 0.f), hand_l, hand_r;
         if (smplx) {
             if (!d.hands_meanl || !d.hands_meanr || !d.hands_componentsl || !d.hands_componentsr || 3 * J < 165) { err = "SMPL-X needs the hand PCA tables"; return false; }
-            for (int i = 0; i < 45; ++i) { pose_mean[75 + i] = d.hands_meanl[i]; pose_mean[120 + i] = d.hands_meanr[i]; }
-            hand_l.assign(d.hands_componentsl, d.hands_componentsl + 6 * 45);
-            hand_r.assign(d.hands_componentsr, d.hands_componentsr + 6 * 45);
+            if (!d.flat_hand_mean)
+                for (int i = 0; i < 45; ++i) { pose_mean[75 + i] = d.hands_meanl[i]; pose_mean[120 + i] = d.hands_meanr[i]; }
+            if (d.hand_axis_angle) {                     // no projection: the identity, so the kernels keep one hand loop
+                hand_l.assign(45 * 45, 0.f);
+                for (int i = 0; i < 45; ++i) hand_l[i * 45 + i] = 1.f;
+                hand_r = hand_l;
+            } else {
+                hand_l.assign(d.hands_componentsl, d.hands_componentsl + (size_t)nhand * 45);
+                hand_r.assign(d.hands_componentsr, d.hands_componentsr + (size_t)nhand * 45);
+            }
         }
 
         // output joint table before the joint map
@@ -558,7 +573,7 @@ struct Builder {
         std::vector<JointEntry> act_table(joint_table.begin(), joint_table.begin() + K_used);
         if (!build_vset(active, act_table, true, &m->act)) return false;
         m->J = J; m->P = P; m->NS = NS; m->NB = NB; m->Kp = Kp; m->NP = NP; m->is_smplx = smplx ? 1 : 0;
-        m->max_depth = max_depth; m->K_used = K_used; m->n_gmm = n_gmm; m->face = face ? 1 : 0;
+        m->max_depth = max_depth; m->K_used = K_used; m->n_gmm = n_gmm; m->face = face ? 1 : 0; m->n_hand = nhand;
         return true;
     }
 };

@@ -5,7 +5,7 @@
 //                      confidences as [N,1], which broadcasts against the [N] residuals, so every joint of such a group
 //                      weighs sum_i conf_i^2 of that group and view (smplify/loss.py:134 with :168,:173,:179).
 //   k_init_theta     : network output (betas [B,10], poses [B,>=3+nbody]) -> theta rows: transl 0, scale 1, global
-//                      orient / body pose / betas from the network, eyes / hands 0 (smplify/smplify.py:103-128).  A model
+//                      orient / body pose / betas from the network, eyes / hands / face 0 (smplify/smplify.py:103-128).  A model
 //                      with more than 10 betas (the kid model) starts the others at 0; one with fewer takes the first NB.
 //   halo             : the temporal term couples frame f with f-1 / f+1; across shards the boundary rows live on the
 //                      neighbouring GPUs.  Each rank owns one small cudaMalloc'ed buffer (exported by CUDA IPC, mapped by
@@ -18,7 +18,8 @@
 #pragma once
 #include "bf_common.cuh"
 
-#define BF_HALO_ROW 128                      // floats per boundary row slot (NP <= 111)
+#define BF_HALO_ROW 128                      // floats per boundary row slot: the first min(NP, 128) theta entries (the
+                                             // temporal term reads transl / global_orient / body_pose, entries below 76)
 #define BF_HALO_PREV 0                       // [2][128] rows written by rank-1 (its LAST frame)
 #define BF_HALO_NEXT (2 * BF_HALO_ROW)       // [2][128] rows written by rank+1 (its FIRST frame)
 #define BF_HALO_FLAGS (4 * BF_HALO_ROW)      // uint32: flag_prev[2], flag_next[2]
@@ -62,8 +63,9 @@ __global__ void __launch_bounds__(64) k_halo_begin(BfFrames f, int NP, int n_ite
     if (threadIdx.x == 0) { base_s = epoch[0] + (uint32_t)n_iters; epoch[0] = base_s; }
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp == 0 && f.halo_peer_prev) halo_push_row(f.theta, NP, f.halo_peer_prev, BF_HALO_NEXT, base_s, lane);
-    if (warp == 1 && f.halo_peer_next) halo_push_row(f.theta + (size_t)(f.B - 1) * NP, NP, f.halo_peer_next, BF_HALO_PREV, base_s, lane);
+    const int nrow = min(NP, BF_HALO_ROW);
+    if (warp == 0 && f.halo_peer_prev) halo_push_row(f.theta, nrow, f.halo_peer_prev, BF_HALO_NEXT, base_s, lane);
+    if (warp == 1 && f.halo_peer_next) halo_push_row(f.theta + (size_t)(f.B - 1) * NP, nrow, f.halo_peer_next, BF_HALO_PREV, base_s, lane);
 }
 
 #define PK_MAXG 4

@@ -7,6 +7,9 @@
 //                Adam update, fused per frame.
 // A face-parameter SMPL-X model (BfModel.face) also carries the jaw pose and the expression coefficients in theta: the forward
 // takes them into the full pose / shape row, the backward produces their gradients (+ the expression L2 prior) and Adam steps them.
+// Hands: n_hand parameters per hand, expanded by the [n_hand,45] component tables (the identity for axis-angle hands).
+// Both kernels are instantiated for two theta capacities per frame: BF_THETA_SMEM (every row of at most 112 entries, the
+// default launch shape) and BF_THETA_SMEM_WIDE (longer rows: wider hands); the launcher picks one from BfModel.NP.
 // Replaces smplx batch_rodrigues + batch_rigid_transform (restated in oracle/smplx_port.py),
 // smplify/prior.py:181-196, smplify/loss.py:54-61,206-217 and torch.optim.Adam
 // (smplify/smplify.py:167-174,211-213).
@@ -17,8 +20,9 @@
 // fp | R | Jr | GR are contiguous and 16-byte aligned (in PoseSmemBwd), in the order of a saved forward-state row ([fp 3J |
 // R 9J | Jr 3J | GR 9J], pose_write_outputs): for J == BF_MAXJ the backward fetches the row with ONE bulk copy.  No tail
 // padding: PoseSmemBwd packs its scratch right behind it (see the size check there).
-struct PoseSmem {
-    float th[BF_THETA_SMEM];
+template <int TH>
+struct PoseSmemT {
+    float th[TH];
     float sh[BF_MAXNS];
     float fp[BF_MAXJ * 3];
     float R[BF_MAXJ * 9];
@@ -26,28 +30,39 @@ struct PoseSmem {
     float GR[BF_MAXJ * 9];
     float Gt[BF_MAXJ * 3];
 };
+typedef PoseSmemT<BF_THETA_SMEM> PoseSmem;
+typedef PoseSmemT<BF_THETA_SMEM_WIDE> PoseSmemWide;
 static_assert((BF_THETA_SMEM + BF_MAXNS) % 4 == 0 && offsetof(PoseSmem, fp) % 16 == 0, "PoseSmem::fp must be 16-byte aligned");
-static_assert(BF_THETA_SMEM >= BF_MAXNP - 9 + BF_MAXNS, "PoseSmem::th must hold the longest face-parameter row");
+static_assert((BF_THETA_SMEM_WIDE + BF_MAXNS) % 4 == 0 && offsetof(PoseSmemWide, fp) % 16 == 0, "PoseSmemWide::fp must be 16-byte aligned");
+static_assert(BF_THETA_SMEM >= BF_MAXNP - 9 + BF_MAXNS, "PoseSmem::th must hold the longest face-parameter row with 6 hand components");
+static_assert(BF_THETA_SMEM_WIDE >= BF_MAXNP - 9 + BF_MAXNS + 2 * (BF_MAXHAND - 6), "PoseSmemWide::th must hold the longest row");
 // Backward scratch.  Everything else the backward needs lives in forward slots that are dead by then (smaller footprint ->
 // six CTAs of four frames per SM): d(posed joints) and later d(rel) in f.Gt (the backward never reads the posed joints),
 // d(full pose) in f.fp (each lane overwrites exactly the three angles it has just consumed), the updated theta in f.th, and --
 // once the reverse chain traversal is done with the local rotations -- the gradient row in f.R[0:NP] and d(rest joints) in
-// f.R[128:128+3J] (until then each lane keeps the d(rest joints) of its own joints in registers).
-struct __align__(16) PoseSmemBwd {
-    PoseSmem f;
+// f.R[dJr_off:dJr_off+3J] (until then each lane keeps the d(rest joints) of its own joints in registers).
+template <int TH>
+struct __align__(16) PoseSmemBwdT {
+    PoseSmemT<TH> f;
     float dGR[BF_MAXJ * 9];
     uint64_t bar;                 // mbarrier of the forward-state bulk copy
+    static constexpr int dJr_off = TH <= 128 ? 128 : TH;   // d(rest joints) in f.R, right behind the gradient row
 };
+typedef PoseSmemBwdT<BF_THETA_SMEM> PoseSmemBwd;
+typedef PoseSmemBwdT<BF_THETA_SMEM_WIDE> PoseSmemBwdWide;
 // 13 CTAs of the default two frames fit into an SM's 228 KB (+ 1 KB per CTA): 2 * 8464 + 1024 = 17952 bytes per CTA.  The
 // face-parameter theta storage (BF_THETA_SMEM) fits into what the 16-byte tail padding of PoseSmem used to take.
 static_assert(sizeof(PoseSmemBwd) <= 8464, "k_pose_bwd: 13 CTAs of 2 frames per SM need <= 8464 bytes per frame");
-static_assert(BF_THETA_SMEM <= 128 && 128 + BF_MAXJ * 3 <= BF_MAXJ * 9, "gradient row / d(rest joints) must fit into PoseSmem::R");
+static_assert(PoseSmemBwd::dJr_off == 128 && PoseSmemBwdWide::dJr_off + BF_MAXJ * 3 <= BF_MAXJ * 9,
+              "gradient row / d(rest joints) must fit into PoseSmem::R");
 
 // Fills S for frame b (all lanes of one warp participate).
-__device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmem& S, int lane);
+template <int TH>
+__device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmemT<TH>& S, int lane);
 
+template <int TH>
 __device__ __forceinline__ void pose_forward_warp(const BfModel& m, const float* __restrict__ theta_row,
-                                                  PoseSmem& S, int lane) {
+                                                  PoseSmemT<TH>& S, int lane) {
     const int np = theta_layout(m).np;
     for (int i = lane; i < np; i += 32) S.th[i] = theta_row[i];
     __syncwarp();
@@ -55,7 +70,8 @@ __device__ __forceinline__ void pose_forward_warp(const BfModel& m, const float*
 }
 
 // theta already in S.th
-__device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmem& S, int lane) {
+template <int TH>
+__device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSmemT<TH>& S, int lane) {
     const ThetaLayout L = theta_layout(m);
     const int J = m.J;
     // full pose
@@ -69,12 +85,10 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
             else if (i < 75) v = S.th[L.off_reye + (i - 72)];
             else if (i < 120) {
                 const int c0 = i - 75;
-#pragma unroll
-                for (int c = 0; c < 6; ++c) v += S.th[L.off_lh + c] * __ldg(m.hand_l + c * 45 + c0);
+                for (int c = 0; c < m.n_hand; ++c) v += S.th[L.off_lh + c] * __ldg(m.hand_l + c * 45 + c0);
             } else {
                 const int c0 = i - 120;
-#pragma unroll
-                for (int c = 0; c < 6; ++c) v += S.th[L.off_rh + c] * __ldg(m.hand_r + c * 45 + c0);
+                for (int c = 0; c < m.n_hand; ++c) v += S.th[L.off_rh + c] * __ldg(m.hand_r + c * 45 + c0);
             }
         }
         S.fp[i] = v + __ldg(m.pose_mean + i);
@@ -147,7 +161,8 @@ __device__ __forceinline__ void pose_forward_from_smem(const BfModel& m, PoseSme
 // forward outputs of frame b from the state in S: GEMM A operand (+ 3xTF32 split), joint transforms,
 // posed joints, full pose, contour-landmark row
 // mask_par: parity of the iteration that will consume these outputs (selects the block-mask buffer, BfFrames.blk_mask)
-__device__ __forceinline__ void pose_write_outputs(const BfModel& m, const BfFrames& f, PoseSmem& S, int b, int lane, int mask_par) {
+template <int TH>
+__device__ __forceinline__ void pose_write_outputs(const BfModel& m, const BfFrames& f, PoseSmemT<TH>& S, int b, int lane, int mask_par) {
     const int J = m.J;
     if (f.fwd_state) {                       // [fp 3J | R 9J | Jr 3J | GR 9J] for the backward pass
         float* st = f.fwd_state + (size_t)b * 24 * J;
@@ -214,13 +229,14 @@ __device__ __forceinline__ void pose_write_outputs(const BfModel& m, const BfFra
     }
 }
 
+template <int TH>
 __global__ void __launch_bounds__(128) k_pose_fwd(BfModel m, BfFrames f) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    PoseSmem* all = reinterpret_cast<PoseSmem*>(smem_raw);
+    PoseSmemT<TH>* all = reinterpret_cast<PoseSmemT<TH>*>(smem_raw);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * (blockDim.x >> 5) + warp;
     if (b >= f.B) return;
-    PoseSmem& S = all[warp];
+    PoseSmemT<TH>& S = all[warp];
     pose_forward_warp(m, f.theta + (size_t)b * m.NP, S, lane);
     pose_write_outputs(m, f, S, b, lane, f.iter & 1);
 }
@@ -233,14 +249,19 @@ struct AdamArgs { float step_ts, step_lr, bc2_sqrt, beta2, om_beta1, om_beta2, e
 
 // (128, 7): at most 72 registers, so that the default launch shape (2 warps per CTA) keeps 13 CTAs per SM, the shared-memory
 // bound; without the cap the face-parameter code paths let ptxas take 96 registers, which would cut it to 10
+// TH: theta capacity per frame.  Up to 128 entries the Adam moments are prefetched into registers at kernel entry (4 per
+// lane); the wide instantiation reads them at the step instead, so that it needs no more registers.
+template <int TH>
 __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int flags, AdamArgs ad) {
+    constexpr bool kPrefetchAdam = TH <= 128;
+    constexpr int kSlots = (TH + 31) / 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    PoseSmemBwd* all = reinterpret_cast<PoseSmemBwd*>(smem_raw);
+    PoseSmemBwdT<TH>* all = reinterpret_cast<PoseSmemBwdT<TH>*>(smem_raw);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * (blockDim.x >> 5) + warp;
     if (b >= f.B) return;
-    PoseSmemBwd& W = all[warp];
-    PoseSmem& S = W.f;
+    PoseSmemBwdT<TH>& W = all[warp];
+    PoseSmemT<TH>& S = W.f;
     float* const drel = S.Gt;
     float* const dfp = S.fp;
     const int J = m.J;
@@ -272,7 +293,7 @@ __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int 
         }
     }
     float am_r[4], av_r[4], gg_r[3];
-    if (flags & 2) {
+    if (kPrefetchAdam && (flags & 2)) {
 #pragma unroll
         for (int s = 0; s < 4; ++s) {
             const int i = lane + 32 * s;
@@ -287,7 +308,7 @@ __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int 
         }
     }
     float* const g = S.R;                    // gradient row: live from the betas phase on (S.R is dead by then)
-    float* const dJr_s = S.R + 128;          // d(rest joints), same
+    float* const dJr_s = S.R + PoseSmemBwdT<TH>::dJr_off;   // d(rest joints), same
     const float g_ts = (lane < 4 && (flags & 4)) ? f.grad[(size_t)b * m.NP + lane] : 0.f;     // d/d(transl, scale) from the loss kernel
     if (f.fwd_state) {                       // forward state saved by the pose forward of this iteration
         for (int i = lane; i < L.np; i += 32) S.th[i] = f.theta[(size_t)b * m.NP + i];
@@ -469,14 +490,17 @@ __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int 
     for (int i = lane; i < 3 + L.nbody; i += 32) g[4 + i] = dfp[i];      // global_orient + body_pose
     if (m.is_smplx) {
         if (lane < 3) { g[L.off_leye + lane] = dfp[69 + lane]; g[L.off_reye + lane] = dfp[72 + lane]; }
-        if (lane < 12) {
-            const int c = lane % 6;
-            const float* comp = (lane < 6 ? m.hand_l : m.hand_r) + c * 45;
-            const float* d = dfp + (lane < 6 ? 75 : 120);
+        // hand parameters: lanes (side, component), 2 n_hand outputs (one pass for up to 16 components per hand)
+        const int nh = m.n_hand;
+        for (int q = lane; q < 2 * nh; q += 32) {
+            const bool left = q < nh;
+            const int c = left ? q : q - nh;
+            const float* comp = (left ? m.hand_l : m.hand_r) + c * 45;
+            const float* d = dfp + (left ? 75 : 120);
             float acc = 0.f;
 #pragma unroll 15
             for (int i = 0; i < 45; ++i) acc += __ldg(comp + i) * d[i];
-            g[(lane < 6 ? L.off_lh : L.off_rh) + c] = acc;
+            g[(left ? L.off_lh : L.off_rh) + c] = acc;
         }
     }
     __syncwarp();
@@ -548,11 +572,13 @@ __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int 
         float* am = f.adam_m + (size_t)b * m.NP;
         float* av = f.adam_v + (size_t)b * m.NP;
 #pragma unroll
-        for (int s = 0; s < 4; ++s) {
+        for (int s = 0; s < kSlots; ++s) {
             const int i = lane + 32 * s;
             if (i >= m.NP) break;
             const float gi = g[i];
-            float mi = am_r[s], vi = av_r[s];              // loaded at kernel entry
+            float mi, vi;
+            if (kPrefetchAdam) { mi = am_r[s & 3]; vi = av_r[s & 3]; }    // loaded at kernel entry
+            else { mi = am[i]; vi = av[i]; }
             mi = mi + (gi - mi) * ad.om_beta1;
             vi = vi * ad.beta2 + ad.om_beta2 * gi * gi;
             const float denom = sqrtf(vi) / ad.bc2_sqrt + ad.eps;
@@ -565,8 +591,9 @@ __global__ void __launch_bounds__(128, 7) k_pose_bwd(BfModel m, BfFrames f, int 
         if ((flags & 16) && f.halo_buf && (b == 0 || b + 1 == f.B)) {
             __syncwarp();
             const uint32_t tick = *reinterpret_cast<const uint32_t*>(f.halo_buf + BF_HALO_EPOCH) + (uint32_t)f.iter + 1u;
-            if (b == 0 && f.halo_peer_prev) halo_push_row(S.th, m.NP, f.halo_peer_prev, BF_HALO_NEXT, tick, lane);
-            if (b + 1 == f.B && f.halo_peer_next) halo_push_row(S.th, m.NP, f.halo_peer_next, BF_HALO_PREV, tick, lane);
+            const int nrow = min(m.NP, BF_HALO_ROW);      // the temporal term reads entries below 7 + nbody only
+            if (b == 0 && f.halo_peer_prev) halo_push_row(S.th, nrow, f.halo_peer_prev, BF_HALO_NEXT, tick, lane);
+            if (b + 1 == f.B && f.halo_peer_next) halo_push_row(S.th, nrow, f.halo_peer_next, BF_HALO_PREV, tick, lane);
         }
         if (flags & 8) {
             __syncwarp();

@@ -32,7 +32,7 @@ from . import constants as K
 
 
 MAX_NS = 20         # betas + expression coefficients per frame (BF_MAXNS, csrc/bf_common.cuh)
-MAX_NP = 100        # theta entries per frame without the face block (BF_MAXNP)
+MAX_NP = 100        # theta entries per frame without the face block, counted with 6 hand components (BF_MAXNP)
 
 
 def _round_up(x, m):
@@ -76,9 +76,10 @@ def load_model_data(path_or_dict, model_type=None, gender='neutral'):
 
 
 def model_desc(smpl_type, data, gmm=None, J_regressor_extra=None, num_betas=10, num_expression=10, tensor_cores=True,
-               gender='neutral', kid_template=None, face_params=False):
+               gender='neutral', kid_template=None, face_params=False, num_pca_comps=6, use_pca=True, flat_hand_mean=False):
     """``(BfModelDesc, keepalive)`` for ``bf_model_create`` / ``bf_model_build_blob``: the raw model arrays as the C ABI
-    takes them (what a non-Python host would pass after reading the model file itself)."""
+    takes them (what a non-Python host would pass after reading the model file itself).  The hand options are passed as
+    given; the C++ builder validates them."""
     data = load_model_data(data, smpl_type, gender)
     keep = []
 
@@ -100,6 +101,7 @@ def model_desc(smpl_type, data, gmm=None, J_regressor_extra=None, num_betas=10, 
     d.is_smplx, d.V, d.J, d.F, d.n_shape_dirs = int(smpl_type == 'smplx'), vt.shape[0], W.shape[1], faces.shape[0], sd.shape[2]
     d.num_betas, d.num_expression, d.tensor_cores = num_betas, num_expression, int(bool(tensor_cores))
     d.face_params = int(bool(face_params))
+    d.num_pca_comps, d.hand_axis_angle, d.flat_hand_mean = int(num_pca_comps), int(not use_pca), int(bool(flat_hand_mean))
     if smpl_type == 'smplx':
         d.hands_meanl, d.hands_meanr = arr(data['hands_meanl'], np.float32), arr(data['hands_meanr'], np.float32)
         d.hands_componentsl, d.hands_componentsr = arr(data['hands_componentsl'], np.float32), arr(data['hands_componentsr'], np.float32)
@@ -123,10 +125,15 @@ class PreparedModel(object):
     """numpy tables -> device tensors -> BfModel struct (kept alive by this object).
 
     ``face_params=True`` (SMPL-X only) builds a face-parameter model: theta rows end with [jaw 3 | expression NE], which the
-    operator takes as inputs and the fit optimises.  Without it the jaw and the expression stay at zero, as in the reference."""
+    operator takes as inputs and the fit optimises.  Without it the jaw and the expression stay at zero, as in the reference.
+
+    Hands (SMPL-X only; smplx.create's options and defaults): ``num_pca_comps`` PCA components per hand (1..45, the first rows
+    of the model's component tables), ``use_pca=False`` for 45 axis-angle entries per hand instead, ``flat_hand_mean=True``
+    to leave the hand mean out of the full pose.  ``n_hand`` is the number of hand parameters per hand in theta."""
 
     def __init__(self, smpl_type, data, gmm=None, J_regressor_extra=None, device='cuda', num_betas=10,
-                 num_expression=10, tensor_cores=None, gender='neutral', age='adult', kid_template=None, face_params=False):
+                 num_expression=10, tensor_cores=None, gender='neutral', age='adult', kid_template=None, face_params=False,
+                 num_pca_comps=6, use_pca=True, flat_hand_mean=False):
         assert smpl_type in ('smpl', 'smplx')
         self.smpl_type = smpl_type
         self.is_smplx = smpl_type == 'smplx'
@@ -150,6 +157,12 @@ class PreparedModel(object):
         if face_params and not self.is_smplx:
             raise ValueError('face parameters (jaw pose, expression) apply to SMPL-X only')
         self.face_params = bool(face_params)
+        if not self.is_smplx and (num_pca_comps != 6 or not use_pca or flat_hand_mean):
+            raise ValueError('hand options (num_pca_comps, use_pca, flat_hand_mean) apply to SMPL-X only')
+        if not 1 <= num_pca_comps <= 45:
+            raise ValueError('num_pca_comps must be between 1 and 45')
+        self.num_pca_comps, self.use_pca, self.flat_hand_mean = int(num_pca_comps), bool(use_pca), bool(flat_hand_mean)
+        self.n_hand = (self.num_pca_comps if self.use_pca else 45) if self.is_smplx else 0
         NB = num_betas
         sd_all = np.asarray(data['shapedirs'], dtype=np.float32)
         if sd_all.ndim == 2:
@@ -181,8 +194,10 @@ class PreparedModel(object):
         if NP > MAX_NP:
             raise ValueError('%d theta entries exceed the limit of %d' % (NP, MAX_NP))
         self.NE = NS - NB
+        if self.is_smplx:
+            NP += 2 * (self.n_hand - 6)             # the limit above counts 6 hand parameters; at most 189 entries
         if self.face_params:
-            NP += 3 + self.NE                       # [jaw 3 | expression NE]; bounded by MAX_NS, at most 111 entries
+            NP += 3 + self.NE                       # [jaw 3 | expression NE]; bounded by MAX_NS
         if self.is_smplx and sd_all.shape[-1] >= K.SHAPE_SPACE_DIM + num_expression:
             # official files: the expression directions follow the 300 shape directions (smplx: SHAPE_SPACE_DIM)
             sd = np.concatenate([sd_all[:, :, :NB], sd_all[:, :, K.SHAPE_SPACE_DIM:K.SHAPE_SPACE_DIM + num_expression]], -1)
@@ -216,10 +231,17 @@ class PreparedModel(object):
         pose_mean = np.zeros(3 * J, dtype=np.float32)
         hand_l = hand_r = None
         if self.is_smplx:
-            pose_mean[75:120] = np.asarray(data['hands_meanl'], dtype=np.float32)
-            pose_mean[120:165] = np.asarray(data['hands_meanr'], dtype=np.float32)
-            hand_l = np.asarray(data['hands_componentsl'], dtype=np.float32)[:6]
-            hand_r = np.asarray(data['hands_componentsr'], dtype=np.float32)[:6]
+            if not self.flat_hand_mean:
+                pose_mean[75:120] = np.asarray(data['hands_meanl'], dtype=np.float32)
+                pose_mean[120:165] = np.asarray(data['hands_meanr'], dtype=np.float32)
+            if self.use_pca:
+                hand_l = np.asarray(data['hands_componentsl'], dtype=np.float32)[:self.n_hand]
+                hand_r = np.asarray(data['hands_componentsr'], dtype=np.float32)[:self.n_hand]
+                if hand_l.shape != (self.n_hand, 45) or hand_r.shape != (self.n_hand, 45):
+                    raise ValueError('num_pca_comps=%d needs at least %d hand component rows of 45 entries (the model has %s / %s)'
+                                     % (self.n_hand, self.n_hand, hand_l.shape, hand_r.shape))
+            else:                                   # axis-angle hands: the identity, so the kernels keep one hand loop
+                hand_l = hand_r = np.eye(45, dtype=np.float32)
 
         # ---- output joint table (pre-map list, then the reference's joint map) --------------------
         # vertex-picked joints: the official files do not list them (smplx hard-codes the ids)
@@ -326,7 +348,8 @@ class PreparedModel(object):
         self._fill_vset(self.struct.full, 'full', full_h)
         self._fill_vset(self.struct.act, 'act', act_h)
         for k, v in dict(J=J, P=P, NS=NS, NB=NB, Kp=self.Kp, NP=self.NP, is_smplx=int(self.is_smplx),
-                         max_depth=self.max_depth, K_used=K_used, n_gmm=self.n_gmm, face=int(self.face_params)).items():
+                         max_depth=self.max_depth, K_used=K_used, n_gmm=self.n_gmm, face=int(self.face_params),
+                         n_hand=self.n_hand).items():
             setattr(self.struct, k, v)
         self.n_act = int(act_h['n'])
         self.n_pad_full = int(full_h['n_pad'])
@@ -550,8 +573,9 @@ class PreparedModel(object):
 
     def pack_theta(self, global_orient, body_pose, betas, transl=None, scale=None, leye=None, reye=None,
                    lhand=None, rhand=None, jaw=None, expression=None):
-        """Assemble [B, NP] theta rows (layout in include/bodyfit_b200.h).  ``jaw`` [B,3] / ``expression`` [B,NE] belong to a
-        face-parameter model (None = 0); a face-off model accepts them only as None."""
+        """Assemble [B, NP] theta rows (layout in include/bodyfit_b200.h).  ``lhand`` / ``rhand`` are [B, n_hand] (PCA
+        coefficients, or 45 axis-angle entries).  ``jaw`` [B,3] / ``expression`` [B,NE] belong to a face-parameter model
+        (None = 0); a face-off model accepts them only as None."""
         B = global_orient.shape[0]
         dev, dt = self.device, torch.float32
         z = lambda n: torch.zeros(B, n, device=dev, dtype=dt)
@@ -562,7 +586,7 @@ class PreparedModel(object):
         parts = [f(transl, 3), torch.ones(B, 1, device=dev, dtype=dt) if scale is None else f(scale, 1),
                  f(global_orient, 3), f(body_pose, self.nbody), bt]
         if self.is_smplx:
-            parts += [f(leye, 3), f(reye, 3), f(lhand, 6), f(rhand, 6)]
+            parts += [f(leye, 3), f(reye, 3), f(lhand, self.n_hand), f(rhand, self.n_hand)]
         if self.face_params:
             parts += [f(jaw, 3), f(expression, self.NE)]
         elif jaw is not None or expression is not None:
@@ -574,9 +598,10 @@ class PreparedModel(object):
         out = dict(transl=theta[:, 0:3], scale=theta[:, 3:4], global_orient=theta[:, 4:7],
                    body_pose=theta[:, 7:7 + nb], betas=theta[:, 7 + nb:7 + nb + self.NB])
         if self.is_smplx:
-            o = 7 + nb + self.NB
+            o, nh = 7 + nb + self.NB, self.n_hand
             out.update(leye_pose=theta[:, o:o + 3], reye_pose=theta[:, o + 3:o + 6],
-                       left_hand_pose=theta[:, o + 6:o + 12], right_hand_pose=theta[:, o + 12:o + 18])
+                       left_hand_pose=theta[:, o + 6:o + 6 + nh], right_hand_pose=theta[:, o + 6 + nh:o + 6 + 2 * nh])
+            o += 6 + 2 * nh
             if self.face_params:
-                out.update(jaw_pose=theta[:, o + 18:o + 21], expression=theta[:, o + 21:o + 21 + self.NE])
+                out.update(jaw_pose=theta[:, o:o + 3], expression=theta[:, o + 3:o + 3 + self.NE])
         return out

@@ -81,17 +81,23 @@ class SMPL(nn.Module):
 class SMPLX(nn.Module):
     """SMPL-X as ``SMPLify.__init__`` builds it: 6 PCA hand components, 10 betas + 10 expression coefficients, contour
     landmarks, joints mapped to the 135 OpenPose keypoints (smplify.py:59-80).  Built as a face-parameter model, so
-    ``forward`` takes ``jaw_pose`` and ``expression`` like ``smplx.SMPLX.forward``, with gradients (None = 0)."""
+    ``forward`` takes ``jaw_pose`` and ``expression`` like ``smplx.SMPLX.forward``, with gradients (None = 0).
+    ``num_pca_comps`` / ``use_pca`` / ``flat_hand_mean`` are smplx's hand options: the hand poses are then
+    [B, num_pca_comps], or [B, 45] axis-angle without PCA."""
 
-    def __init__(self, model_data, device='cuda', num_betas=10, num_expression=10, **kwargs):
+    def __init__(self, model_data, device='cuda', num_betas=10, num_expression=10, num_pca_comps=6, use_pca=True,
+                 flat_hand_mean=False, **kwargs):
         super().__init__()
         self.prepared = PreparedModel('smplx', model_data, gmm=None, device=device, num_betas=num_betas,
-                                      num_expression=num_expression, face_params=True)
+                                      num_expression=num_expression, face_params=True, num_pca_comps=num_pca_comps,
+                                      use_pca=use_pca, flat_hand_mean=flat_hand_mean)
         self.faces = self.prepared.faces
+        self.num_pca_comps, self.use_pca, self.flat_hand_mean = num_pca_comps, use_pca, flat_hand_mean
 
     def forward(self, global_orient=None, body_pose=None, betas=None, jaw_pose=None, leye_pose=None, reye_pose=None,
                 left_hand_pose=None, right_hand_pose=None, expression=None, return_full_pose=False, **kwargs):
-        """``jaw_pose`` [B,3] or [B,1,3], ``expression`` [B,NE]; both differentiable, None = 0."""
+        """``jaw_pose`` [B,3] or [B,1,3], ``expression`` [B,NE], ``left_hand_pose`` / ``right_hand_pose`` [B, n_hand]
+        (``prepared.n_hand``: num_pca_comps, or 45 without PCA); all differentiable, None = 0."""
         pm = self.prepared
         theta = pm.pack_theta(global_orient, body_pose, betas, leye=leye_pose, reye=reye_pose, lhand=left_hand_pose,
                               rhand=right_hand_pose, jaw=jaw_pose, expression=expression)
@@ -102,7 +108,8 @@ class SMPLX(nn.Module):
 
 
 def create_smplx(model_path='data', gender='neutral', model_data=None, device='cuda', num_betas=10, num_expression=10,
-                 **kwargs):
+                 num_pca_comps=6, use_pca=True, flat_hand_mean=False, **kwargs):
     from ..model import load_model_data
     data = model_data if model_data is not None else load_model_data(model_path, 'smplx', gender)
-    return SMPLX(data, device=device, num_betas=num_betas, num_expression=num_expression)
+    return SMPLX(data, device=device, num_betas=num_betas, num_expression=num_expression, num_pca_comps=num_pca_comps,
+                 use_pca=use_pca, flat_hand_mean=flat_hand_mean)

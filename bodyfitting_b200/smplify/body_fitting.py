@@ -20,7 +20,9 @@ class BodyFitting(object):
     def __init__(self, options=None, smpl_type=None, age='adult', use_mask=False, debug=False, init_fn=None, regressor=None,
                  face_params=False, **smplify_kw):
         """``face_params=True`` (SMPL-X): the fits also optimise jaw pose and expression (SMPLify(face_params=)); the results
-        and the saved parameter file then hold ``jaw_pose`` and ``expression``."""
+        and the saved parameter file then hold ``jaw_pose`` and ``expression``.  The hand options ``num_pca_comps``,
+        ``use_pca`` and ``flat_hand_mean`` pass through ``smplify_kw`` to SMPLify (or come from ``options``); the saved
+        hand poses then have num_pca_comps (or 45) entries."""
         self.options = options
         self.smpl_type = smpl_type or getattr(options, 'smpl_type', 'smpl')
         self.age = getattr(options, 'age', age)
@@ -30,6 +32,9 @@ class BodyFitting(object):
         self.init_fn = init_fn
         self.regressor = regressor
         self.face_params = bool(getattr(options, 'face_params', face_params))
+        for k in ('num_pca_comps', 'use_pca', 'flat_hand_mean'):
+            if hasattr(options, k):
+                smplify_kw.setdefault(k, getattr(options, k))
         self.smplify_kw = smplify_kw
         self._smplify = {}
 
@@ -68,7 +73,8 @@ class BodyFitting(object):
 
 def write_result(output_folder, smpl_type, result, disp=False):
     """``{smpl_type}_parameter.npy`` (pickled dict) + ``{smpl_type}.obj`` (+ ``{smpl_type}+d.obj``), body_fitting.py:94-99.
-    The parameter file holds every key of ``result``: ``jaw_pose`` / ``expression`` too when the fit optimised them."""
+    The parameter file holds every key of ``result``: ``jaw_pose`` / ``expression`` too when the fit optimised them, and
+    the hand poses with as many entries as the fit's hand configuration has (num_pca_comps, or 45 without PCA)."""
     os.makedirs(output_folder, exist_ok=True)
     np.save(os.path.join(output_folder, '%s_parameter.npy' % smpl_type), result)
     save_obj_mesh(os.path.join(output_folder, '%s.obj' % smpl_type), result['vertices'], result['faces'])

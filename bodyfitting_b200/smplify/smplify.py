@@ -36,10 +36,13 @@ class SMPLify(object):
                  model_data=None, gmm=None, J_regressor_extra=None, data_root='data', dense_every_iter=False,
                  concurrent_parts=None, concurrent_min_part=512, temporal_weight=0.0, halo_exchange=None, halo=None,
                  copy_outputs=None, graph=None, sort_frames=None, kid_template=None, face_params=False,
-                 expr_prior_weight=K.EXPR_PRIOR_WEIGHT):
+                 expr_prior_weight=K.EXPR_PRIOR_WEIGHT, num_pca_comps=6, use_pca=True, flat_hand_mean=False):
         """``face_params=True`` (SMPL-X only): the fit also optimises the jaw pose and the expression coefficients, with the
         expression prior ``expr_prior_weight^2 * sum psi^2`` (the reference optimises neither, smplify.py:118,167-173; no jaw
-        prior).  The result dict then also holds ``jaw_pose`` and ``expression``."""
+        prior).  The result dict then also holds ``jaw_pose`` and ``expression``.
+        ``num_pca_comps`` / ``use_pca`` / ``flat_hand_mean`` (SMPL-X only; smplx.create's hand options, defaults as in the
+        reference): the fitted ``left_hand_pose`` / ``right_hand_pose`` are then [B, num_pca_comps], or [B, 45] axis-angle
+        without PCA.  Hands step with Adam at the default lr and have no prior, as in the reference."""
         if age not in ('adult', 'kid'):
             raise ValueError("age must be 'adult' or 'kid' (smplify.py:23,112-115)")
         if age == 'kid' and smpl_type != 'smpl':
@@ -71,7 +74,8 @@ class SMPLify(object):
             kid_template = os.path.join(data_root, 'smil', 'smil_web.pkl')           # config.SMIL_MODEL_DIR (config.py:5)
         self.model = PreparedModel(smpl_type, model_data, gmm=gmm, J_regressor_extra=J_regressor_extra,
                                    device=self.device, gender=gender, age=age, kid_template=kid_template,
-                                   face_params=self.face_params)
+                                   face_params=self.face_params, num_pca_comps=num_pca_comps, use_pca=use_pca,
+                                   flat_hand_mean=flat_hand_mean)
         self.smpl_faces = self.model.faces.astype(np.int32).reshape(1, -1, 3)
         self.last_trace = None
         self.dense_every_iter = dense_every_iter

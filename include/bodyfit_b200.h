@@ -24,10 +24,13 @@
  * All floating point data is fp32, row-major, contiguous unless a leading dimension
  * is given.  "theta" is the per-frame optimisation vector:
  *   [transl 3 | scale 1 | global_orient 3 | body_pose 69(smpl) or 63(smplx) | betas 10 |
- *    (smplx only) leye 3 | reye 3 | left_hand_pca 6 | right_hand_pca 6 |
- *    (face-parameter smplx model only, BfModel.face) jaw 3 | expression NE]   NP = 86 / 98 / 98 + 3 + NE
- * with 10 betas (num_betas in general; 11 for the kid model).  The face block of a face-parameter model
- * (BfModelDesc.face_params) follows every other entry, so all other offsets are the same with and without it.
+ *    (smplx only) leye 3 | reye 3 | left_hand nh | right_hand nh |
+ *    (face-parameter smplx model only, BfModel.face) jaw 3 | expression NE]   NP = 86 / 98 / 86 + 2 nh (+ 3 + NE)
+ * with 10 betas (num_betas in general; 11 for the kid model).  nh = BfModel.n_hand: the number of hand PCA components
+ * (6 by default, BfModelDesc.num_pca_comps), or 45 axis-angle entries per hand without PCA (BfModelDesc.hand_axis_angle).
+ * The face block of a face-parameter model (BfModelDesc.face_params) follows every other entry, so all other offsets are
+ * the same with and without it; every offset before left_hand is the same for every hand configuration.  The longest row
+ * (axis-angle hands and face parameters) has 7 + 63 + 10 + 6 + 90 + 3 + 10 = 189 entries.
  */
 #ifndef BODYFIT_B200_H
 #define BODYFIT_B200_H
@@ -43,7 +46,7 @@ extern "C" {
 #define BF_ECUDA    -2   /* a CUDA runtime call / launch failed            */
 #define BF_EARCH    -3   /* device is not sm_100 (no fallback exists)      */
 
-#define BF_ABI_VERSION 20
+#define BF_ABI_VERSION 21
 #define BF_F_WORLD 1   /* forward outputs in world space: (x + transl) * scale * constant_scale */
 #define BF_F_TC    2   /* run the blend-shape contractions on tcgen05 tensor cores (3xTF32) */
 #define BF_F_SKIN_FUSED 4  /* bf_frame_loss_backward skins the frame's live vertices itself from vposed (after bf_blend_forward) */
@@ -100,8 +103,8 @@ typedef struct BfModel {
     const float*   Jt;        /* [J,3]     J_regressor @ v_template */
     const float*   Jd;        /* [J,3,NS]  J_regressor @ shapedirs  */
     const float*   pose_mean; /* [3J] */
-    const float*   hand_l;    /* [6,45] or NULL */
-    const float*   hand_r;    /* [6,45] or NULL */
+    const float*   hand_l;    /* [n_hand,45] hand components (the identity for axis-angle hands) or NULL */
+    const float*   hand_r;    /* [n_hand,45] or NULL */
     const float*   gmm_mean;  /* [8,69] */
     const float*   gmm_psym;  /* [8,69,72] (P + P^T)/2 of each component, rows padded with zeros to 72 */
     const float*   gmm_logw;  /* [8] log(nll_weights) */
@@ -111,7 +114,7 @@ typedef struct BfModel {
     BfVSet act;
     int32_t J, P, NS, NB, Kp, NP, is_smplx, max_depth, K_used, n_gmm;
     int32_t face;             /* 1 = face-parameter SMPL-X model: theta carries jaw pose + the NS - NB expression coefficients */
-    int32_t _pad1;
+    int32_t n_hand;           /* SMPL-X: hand parameters per hand in theta (num_pca_comps, or 45 for axis-angle hands); 0 for SMPL */
 } BfModel;
 
 /* Per-call frame buffers (all device memory, B frames). */
@@ -250,7 +253,8 @@ typedef struct BfModelDesc {
     const int32_t* faces;                   /* [F,3] (SMPL-X: needed for the landmark tables) */
     const float*   hands_meanl;             /* [45]   SMPL-X */
     const float*   hands_meanr;             /* [45] */
-    const float*   hands_componentsl;       /* [>=6,45]: the first six PCA rows are used (smplx num_pca_comps=6) */
+    const float*   hands_componentsl;       /* [>=num_pca_comps,45]: the first num_pca_comps PCA rows are used (unused for
+                                               axis-angle hands) */
     const float*   hands_componentsr;
     const int32_t* lmk_faces_idx;           /* [n_lmk]   SMPL-X static face landmarks */
     const float*   lmk_bary_coords;         /* [n_lmk,3] */
@@ -265,9 +269,15 @@ typedef struct BfModelDesc {
     /* num_betas >= 1 (the kid template adds one more); num_expression >= 0 (SMPL-X only; 0 = no expression directions).
      * The model is rejected when betas + expression exceed 20 or its theta row without the face block exceeds 100 entries
      * (NP above).  face_params != 0 (SMPL-X only): theta also carries the jaw pose and the expression coefficients, which the
-     * fit then optimises (at most 91 + 20 = 111 entries); 0 keeps them at zero, as the reference does. */
+     * fit then optimises; 0 keeps them at zero, as the reference does.
+     * Hands (SMPL-X only, smplx.create's options): num_pca_comps = hand PCA components per hand, 1..45 (0 means 6, the
+     * reference's configuration); the 100-entry limit above is computed with 6.  hand_axis_angle != 0 (smplx use_pca=False):
+     * theta carries 45 axis-angle entries per hand and num_pca_comps is only range-checked.  flat_hand_mean != 0: the hand
+     * mean is not added to the full pose.  Both flags follow the 16 int32 members of ABI 20, so a host that zero-initialises
+     * the struct and fills those keeps its meaning. */
     int32_t is_smplx, V, J, F, n_shape_dirs, num_betas, num_expression, n_lmk, n_dyn_rows, n_dyn, n_extra_vids, n_regressor_extra,
-            n_gmm, tensor_cores, face_params, _pad1;
+            n_gmm, tensor_cores, face_params, num_pca_comps;
+    uint32_t hand_axis_angle, flat_hand_mean;
 } BfModelDesc;
 int     bf_model_create(const BfModelDesc* desc, BfModel** out);
 int     bf_model_build_blob(const BfModelDesc* desc, void** blob, int64_t* nbytes);
@@ -289,7 +299,7 @@ int bf_graph_set_kernel_priority(void* cuda_graph, int priority);
 int bf_pack_keypoints(const float* kp_raw, float* kp_packed, int B, int Nv, int K, int hand_face, const int32_t* src_index,
                       void* stream);
 /* network output -> initial theta rows (smplify/smplify.py:103-128): transl 0, scale 1, global_orient / body_pose from
- * poses[b, 0:3+nbody] (row stride ld_poses), betas[b, 0:10], eye / hand parameters 0.  betas always has 10 columns: a model
+ * poses[b, 0:3+nbody] (row stride ld_poses), betas[b, 0:10], eye / hand (and face) parameters 0.  betas always has 10 columns: a model
  * with more betas (num_betas > 10, the kid model) starts the betas beyond the 10th at 0, one with fewer takes the first
  * num_betas columns.  To start them elsewhere, write the theta rows directly (layout at the top of this file). */
 int bf_init_theta(const BfModel* m, const float* poses, int ld_poses, const float* betas, float* theta, int B,
