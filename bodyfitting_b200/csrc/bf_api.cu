@@ -772,9 +772,18 @@ int bf_pack_keypoints(const float* kp_raw, float* kp_packed, int B, int Nv, int 
                       void* stream) {
     BF_NVTX();
     BF_REQUIRE(kp_raw && kp_packed && B > 0 && Nv > 0 && K > 0, "bad arguments");
+    BF_REQUIRE(Nv <= BF_MAXVIEWS, "Nv out of range (1 to 64 views)");
     BF_REQUIRE(!hand_face || K > 67, "hand / face groups need the SMPL-X joint layout (K > 67)");
+    // one frame's detections + group weights per CTA: 50,720 bytes at 31 SMPL-X views, 104,704 at 64 -- above the 48 KB
+    // default the kernel opts in to more dynamic shared memory
     const size_t smem = sizeof(float) * (((size_t)Nv * K * 3 + 3) / 4 * 4 + (size_t)Nv * PK_MAXG);
-    BF_REQUIRE(smem <= 48 * 1024, "Nv * K too large for one frame per CTA");
+    if (smem > 48 * 1024) {
+        int optin = 0;
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, bf_cur_dev());
+        BF_REQUIRE(smem <= (size_t)optin, "Nv * K too large for one frame per CTA (shared memory of the device)");
+        static size_t attr[BF_MAXDEV] = {0};
+        const int rc = bf_ensure_smem(k_pack_keypoints, smem, attr, "k_pack_keypoints"); if (rc) return rc;
+    }
     k_pack_keypoints<<<B, 256, smem, (cudaStream_t)stream>>>(kp_raw, kp_packed, B, Nv, K, hand_face, src_index);
     BF_LAUNCH_CHECK();
     return BF_OK;

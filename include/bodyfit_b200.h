@@ -170,7 +170,7 @@ typedef struct BfFrames {
                                    move); the 13 KB keypoint rows stay where they are behind this index */
     int64_t      ws_floats;
     double lr_ts, lr, beta1, beta2, eps;   /* Adam hyper-parameters (python floats in the reference: smplify.py:167-174) */
-    int32_t B, Nv, ld_v, iter;
+    int32_t B, Nv, ld_v, iter; /* Nv: camera views, 1 to 64 */
     int32_t flags;             /* BF_F_WORLD: skin/joints forward write (x + transl) * scale * constant_scale (smplify.py:189-190) */
     int32_t halo_iters;        /* NVLink halo: iterations of the run; iteration `iter` publishes its updated boundary rows iff iter + 1 < halo_iters */
     float imsize, constant_scale, sigma, w_pose, w_angle, w_shape;
@@ -295,7 +295,8 @@ int bf_graph_set_kernel_priority(void* cuda_graph, int priority);
 
 /* ---- input packing (so that no host-framework arithmetic sits on the path) ---------------------------------
  * detections [B,Nv,K,3] (x, y, conf) in the caller's layout -> kp [B,K,Nv,3] (x, y, effective weight): conf^2 for the body,
- * the group's sum of conf^2 for SMPL-X hands / face (smplify/loss.py:134 with :168,:173,:179) */
+ * the group's sum of conf^2 for SMPL-X hands / face (smplify/loss.py:134 with :168,:173,:179).  Nv: 1 to 64 views
+ * (BfFrames.Nv); one frame's K * Nv detections are staged in shared memory (at most 104,704 bytes: SMPL-X, 64 views) */
 int bf_pack_keypoints(const float* kp_raw, float* kp_packed, int B, int Nv, int K, int hand_face, const int32_t* src_index,
                       void* stream);
 /* network output -> initial theta rows (smplify/smplify.py:103-128): transl 0, scale 1, global_orient / body_pose from

@@ -134,11 +134,14 @@ def test_lbs_backward_operator(assets, mt):
         assert e < 1e-4, k
 
 
-@pytest.mark.parametrize('mt,nv,B', [('smpl', 4, 6), ('smplx', 8, 4), ('smpl', 5, 3), ('smplx', 3, 2)])
+@pytest.mark.parametrize('mt,nv,B', [('smpl', 4, 6), ('smplx', 8, 4), ('smpl', 5, 3), ('smplx', 3, 2),
+                                     ('smplx', 31, 2), ('smplx', 48, 2), ('smpl', 48, 3)])
 def test_fit_trajectory(assets, mt, nv, B):
     """100 iterations through the drop-in SMPLify class vs the batched oracle loop.  The odd view counts take the
     per-frame kernel's plain-load variant (keypoint rows that are not 16-byte granular cannot be fetched by bulk copy)
-    and its scalar keypoint reads; 4 / 8 views take the TMA-staged variant."""
+    and its scalar keypoint reads; 4 / 8 views take the TMA-staged variant.  SMPL-X at 31 and 48 views stages more than
+    48 KB of detections per frame in the input packing (k_pack_keypoints) and, its keypoint row too large to stage, runs the
+    plain-load variant with 16-byte reads at 48 views; SMPL at 48 views stages its row by bulk copy."""
     from bodyfitting_b200.smplify.smplify import SMPLify
     port = make_port(assets, mt)
     sc = make_scene(port, mt, B, nv, seed=2)
@@ -422,8 +425,13 @@ def test_pack_kernels_match_host_packing(assets):
     """bf_pack_keypoints / bf_init_theta (the input packing of a fit) against the torch / numpy packing of engine.py."""
     from bodyfitting_b200 import _lib
     from bodyfitting_b200.engine import pack_keypoints
-    for mt, nv in (('smplx', 8), ('smpl', 3)):
-        pm = _prep(assets, mt)
+    # 1 to 64 views; SMPL-X from 31 views on stages more than 48 KB of detections per frame (104,704 bytes at 64)
+    pms = {}
+    for mt, nv in (('smplx', 8), ('smpl', 3), ('smplx', 1), ('smplx', 30), ('smplx', 31), ('smplx', 48), ('smplx', 64),
+                   ('smpl', 4), ('smpl', 48), ('smpl', 64)):
+        if mt not in pms:
+            pms[mt] = _prep(assets, mt)
+        pm = pms[mt]
         B, K = 7, pm.K_used
         rng = np.random.RandomState(3)
         kp = torch.from_numpy(rng.rand(B, nv, K, 3).astype(np.float32)).cuda()
@@ -448,6 +456,8 @@ def test_pack_kernels_match_host_packing(assets):
         back = torch.empty_like(theta)
         _lib.check(L.bf_scatter_rows(theta.data_ptr(), idx.data_ptr(), back.data_ptr(), B, pm.NP, st), 'bf_scatter_rows')
         assert torch.equal(back, want_theta)
+    with pytest.raises(_lib.BodyfitError, match='Nv out of range'):
+        _lib.check(L.bf_pack_keypoints(kp.data_ptr(), got.data_ptr(), 1, 65, 25, 0, None, st), 'bf_pack_keypoints')
 
 
 def test_nvlink_halo_shards_of_one_gpu(assets):
